@@ -16,6 +16,10 @@ argmin for one instance (reference: augmented.py:10-87 + horizon_selection.py:36
 
 Launch: `python bench.py --gpus 1 --steps K --warmup W`, or under torchrun for N > 1 (one rank per
 GPU; the batch is sharded, no collective on the solve path, a final all_gather of T*/J*).
+`--dump-outputs DIR` writes what the last timed kernel step returned (rank 0's shard) as float64 .npy files, so that two
+builds can be compared output for output: the inputs depend only on --batch and the rank.
+The benchmark writes nothing into the source tree (which may be read-only): the libraries are built by
+__graft_entry__.build() beforehand.
 """
 from __future__ import annotations
 
@@ -29,6 +33,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True                          # no __pycache__ in the source tree
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "time-opt-ilqr_b200"))
 os.environ.setdefault("OPENBLAS_NUM_THREADS", "1")
@@ -40,6 +45,8 @@ WORKLOAD = ("S1 quadrotor n=12 m=4 d=13 N=128 T in [40,128]: iteration-0 HOP hor
             "(rollout + forward-FD linearisation -> augmented embedding + LFT stage/prefix/query sweep + argmin)")
 UNIT = "solves/s"
 N_HORIZON, D_AUG, M_CTRL = 128, 13, 4
+DUMP_INSTANCES = 1 << 20     # --dump-outputs: per-instance arrays in full up to this batch (8 MiB each)
+DUMP_J_ROWS = 16384          # --dump-outputs: rows of the J(T) curves (16 MiB at T_max = 128; all of them are 64 MiB at the default batch)
 
 
 def f_alg(N, d, m):
@@ -56,6 +63,23 @@ def s1_x0(B, seed):
     x0 = np.zeros(12); x0[:3] = 2.0
     sigma = np.array([0.4, 0.4, 0.4] + [0.0] * 9)
     return x0[None] + sigma[None] * np.random.default_rng(seed).standard_normal((B, 12))
+
+
+def dump_outputs(out_dir, res):
+    """Write a Selection as float64 DIR/<name>.npy: T_star, J_star, status per instance and J, the curves J(T) of a fixed,
+    seeded sample of instances; instances.npy and J_rows.npy hold the batch indices of those rows (at most 48.1 MiB)."""
+    os.makedirs(out_dir, exist_ok=True)
+    B = res.T_star.shape[0]
+
+    def sample(k):
+        return np.arange(B) if B <= k else np.sort(np.random.default_rng(0).choice(B, k, replace=False))
+
+    inst, rows = sample(DUMP_INSTANCES), sample(DUMP_J_ROWS)
+    host = {k: getattr(res, k).cpu().numpy() for k in ("J", "T_star", "J_star", "status")}
+    arrays = {"T_star": host["T_star"][inst], "J_star": host["J_star"][inst], "status": host["status"][inst],
+              "instances": inst, "J": host["J"][rows], "J_rows": rows}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 class ClockSampler:
@@ -115,10 +139,8 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    import oracle as O
     from oracle import ref_py
     from hop import cases
-    O.build()
     case = cases.make_case("Quadrotor", N=N_HORIZON)
     cores = os.cpu_count() or 1
     # ---- the C port: calibrate, then ~2 s of CPU work
@@ -238,6 +260,8 @@ def run_hop(args):
     ms_total = float(ms.item())
     clocks = sampler.stop(tw0, tw1) if rank == 0 else None
     assert torch.equal(r.T_star, T_ref), "kernel-only and from-x0 selections disagree"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r)
     value = world * B * args.steps / (ms_total * 1e-3)
 
     # ---- end-to-end through the public host-buffer API
@@ -304,9 +328,7 @@ def run_hop(args):
         #  * HOP_MODE_EXACT on the same batch on the device: the measured mode against the parity mode
         #  * the REAL reference (oracle/_ref, unmodified Python) on the first instances: T* equality and solves/s per core
         #  * the committed reference-generated golden (first 4096 instances of this very batch, tests/golden)
-        import oracle as O
         from oracle import census, ref_py
-        O.build()
         cores = os.cpu_count() or 1
         t0c = time.perf_counter()
         rep = census.census_from_x0(case, x0_np, J_h, T_h, nthreads=cores, fp80_stride=8)
@@ -399,7 +421,13 @@ def main():
                     help="skip the CPU baseline / parity census (they fork worker processes); only for the ncu launch list")
     ap.add_argument("--ref-kind", choices=["auto", "port"], default="auto",
                     help="--impl reference: auto = the Python reference from oracle/_ref when staged, else the C port")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's T*, J*, status and a seeded sample of J(T) rows to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "hop":
+        ap.error("--dump-outputs applies to --impl hop (the reference arm's sample size is calibrated per run)")
     if args.impl == "reference":
         run_reference(args)
     else:

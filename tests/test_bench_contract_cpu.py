@@ -31,6 +31,13 @@ def test_reference_arm_prints_one_contract_line(ref_kind):
     assert "workload" in d["config"] and d["dtype"] == "f64" and d["data"] == "synthetic"
 
 
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_arguments_it_cannot_honour(extra, tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=600,
+                         cwd=tmp_path)
+    assert out.returncode == 2 and "error:" in out.stderr and not os.listdir(tmp_path)
+
+
 def test_hop_arm_refuses_to_run_without_a_device():
     """No CPU fallback: on a box without CUDA the product arm must fail loudly (skipped where a GPU is present)."""
     import torch
