@@ -218,7 +218,8 @@ int hop_backward_linesearch_f64(int B, int sys, const double *params_host, int N
                                 double *U_new, double *J_new, int *accepted, void *stream);
 
 /* solver.py:233-286 forward_linesearch_fixedT alone, with caller-provided gains k_list [B][N][m],
- * K_list [B][N][m][n] (rows >= T_star[b] ignored); ok [B] or NULL masks instances to skip. */
+ * K_list [B][N][m][n] (rows >= T_star[b] ignored); ok [B] or NULL masks instances to skip: a skipped instance gets
+ * accepted[b] = 0 and keeps X_new, U_new and J_new as the caller left them. */
 int hop_linesearch_f64(int B, int sys, const double *params_host, int N, const double *X, const double *U, const double *xg,
                        const double *w, const double *u_ref, const double *Q, const double *R, const double *Qf,
                        unsigned wrap_mask, const int *T_star, const double *k_list, const double *K_list, const int *ok,

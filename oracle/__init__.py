@@ -258,23 +258,36 @@ def build_terminal(X, xg, alpha, wrap_idx=None, rho_reg=1e-12):
     Qf = _d(as_terminal_weight(alpha, n))
     xg = _d(xg)
     QT = np.empty((N, n + 1, n + 1))
-    lib().hopo_build_terminal(n, N, _p(X), _p(xg), _p(Qf), C.c_uint(wrap_mask(wrap_idx)), C.c_double(rho_reg), _p(QT))
+    rc = lib().hopo_build_terminal(n, N, _p(X), _p(xg), _p(Qf), C.c_uint(wrap_mask(wrap_idx)), C.c_double(rho_reg),
+                                   _p(QT))
+    _raise(rc, "build_terminal")
     return QT
 
 
 # ----------------------------------------------------------------------------- horizon_selection.py
+def _rinv_stride(R_inv, per_step_ndim, N, m):
+    """0 for one R^-1 ([m,m] / [B,m,m]), m*m for one per step ([N,m,m] / [B,N,m,m]: chol_inv(R_list[k]))."""
+    if R_inv.ndim == per_step_ndim:
+        if R_inv.shape[-3] != N:
+            raise ValueError(f"per-step R_inv has {R_inv.shape[-3]} steps, expected N = {N}")
+        return m * m
+    return 0
+
+
 def propagator_all_Jt(A_aug, B_aug, Q_aug, R_inv, z0, QT, T_use=None, f80=False, jitter=1e-9, max_tries=8,
                       return_retries=False):
+    """R_inv: [m,m] (the R_inv_cached argument) or [N,m,m] (chol_inv(R_list[k]) per step)."""
     A_aug, B_aug, Q_aug, QT = _d(A_aug), _d(B_aug), _d(Q_aug), _d(QT)
     R_inv, z0 = _d(R_inv), _d(z0)
     N, d = A_aug.shape[0], A_aug.shape[1]
     m = B_aug.shape[2]
+    stride = _rinv_stride(R_inv, 3, N, m)
     T = N if T_use is None else int(T_use)
     J = np.zeros(max(T, 0))
     retries = (C.c_long * 5)()
     fn = lib().hopo_propagator_all_Jt_f80 if f80 else lib().hopo_propagator_all_Jt_f64
-    rc = fn(T, d, m, _p(A_aug), _p(B_aug), _p(Q_aug), _p(R_inv), _p(z0), _p(QT), _p(J), C.c_double(jitter),
-            int(max_tries), retries)
+    rc = fn(T, d, m, _p(A_aug), _p(B_aug), _p(Q_aug), _p(R_inv), C.c_long(stride), _p(z0), _p(QT), _p(J),
+            C.c_double(jitter), int(max_tries), retries)
     _raise(rc, "chol_inv(A)")
     return (J, list(retries)) if return_retries else J
 
@@ -285,13 +298,17 @@ def argmin_window(J, T_min, T_max):
 
 
 def propagator_batch(A_aug, B_aug, Q_aug, R_inv, z0, QT, T_use=None, nthreads=1):
-    A_aug, B_aug, Q_aug, QT, R_inv, z0 = _d(A_aug), _d(B_aug), _d(Q_aug), _d(QT), _d(R_inv), _d(z0)
+    """R_inv: [m,m] (shared), [B,m,m] (one per instance) or [B,N,m,m] (one per instance and step)."""
+    A_aug, B_aug, Q_aug, QT, z0 = _d(A_aug), _d(B_aug), _d(Q_aug), _d(QT), _d(z0)
     Bsz, N, d = A_aug.shape[0], A_aug.shape[1], A_aug.shape[2]
     m = B_aug.shape[3]
+    R_inv = np.asarray(R_inv, dtype=float)
+    R_inv = _d(np.broadcast_to(R_inv, (Bsz, m, m)) if R_inv.ndim == 2 else R_inv)
+    stride = _rinv_stride(R_inv, 4, N, m)
     T = N if T_use is None else int(T_use)
     J = np.zeros((Bsz, T)); status = np.zeros(Bsz, dtype=np.int32)
     rc = lib().hopo_propagator_batch(int(nthreads), Bsz, N, T, d, m, _p(A_aug), _p(B_aug), _p(Q_aug), _p(R_inv),
-                                     _p(z0), _p(QT), _p(J), _pi(status))
+                                     C.c_long(stride), _p(z0), _p(QT), _p(J), _pi(status))
     _raise(rc, "propagator_batch")
     return J, status
 

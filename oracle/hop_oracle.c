@@ -13,7 +13,10 @@
 
 #define HOP_MAXD 16
 #define HOP_MAXN 16 /* max state dim */
-#define HOP_MAXM 8  /* max control dim */
+#define HOP_MAXM 16 /* max control dim */
+
+/* state / control dimensions an entry point can hold in its stack arrays (the augmented d = n + 1 <= HOP_MAXD) */
+static int dims_ok(int n, int m) { return n >= 1 && n + 1 <= HOP_MAXD && m >= 1 && m <= HOP_MAXM; }
 
 /* ------------------------------------------------------------------------------------------ */
 /* precision-generic linear algebra + propagator                                               */
@@ -216,6 +219,7 @@ double hopo_cost_timeopt_true(int n, int m, const double *X, const double *U, co
                               const double *u_ref, const double *Q, const double *R, const double *Qf,
                               double w, int T_star, unsigned wrap_mask)
 {
+    if (!dims_ok(n, m)) return NAN;
     if (T_star <= 0) return INFINITY;
     if (!vec_finite((T_star + 1) * n, X) || !vec_finite(T_star * m, U)) return INFINITY;
     double c = 0.0, e[HOP_MAXN], du[HOP_MAXM];
@@ -302,6 +306,7 @@ int hopo_build_augmented(int n, int m, int N, const double *A, const double *B, 
                          double rho_reg, double *A_aug, double *B_aug, double *Q_aug, double *R_inv)
 {
     const int d = n + 1;
+    if (!dims_ok(n, m)) return HOP_ERR_ARG;
     double Rs[HOP_MAXM * HOP_MAXM], Qs[HOP_MAXN * HOP_MAXN];
     la_sym_f64(m, R, Rs);
     int rc = la_chol_inv_f64(m, Rs, R_inv, HOP_JITTER, HOP_TRIES, NULL); /* :23 */
@@ -349,10 +354,11 @@ int hopo_build_augmented(int n, int m, int N, const double *A, const double *B, 
 }
 
 /* augmented.py:63-87  build_terminal_aug_list: QT[t-1] from X[t], t = 1..N */
-void hopo_build_terminal(int n, int N, const double *X, const double *xg, const double *Qf,
-                         unsigned wrap_mask, double rho_reg, double *QT)
+int hopo_build_terminal(int n, int N, const double *X, const double *xg, const double *Qf,
+                        unsigned wrap_mask, double rho_reg, double *QT)
 {
     const int d = n + 1;
+    if (!dims_ok(n, 1)) return HOP_ERR_ARG;
     double P[HOP_MAXN * HOP_MAXN];
     la_sym_f64(n, Qf, P);
     for (int t = 1; t <= N; ++t) {
@@ -375,21 +381,24 @@ void hopo_build_terminal(int n, int N, const double *X, const double *xg, const 
         Qt[n * d + n] = 2.0 * p0 + rho_reg;
         la_sym_f64(d, Qt, QT + (size_t)(t - 1) * d * d);
     }
+    return HOP_OK;
 }
 
 int hopo_propagator_all_Jt_f64(int T_use, int d, int m, const double *A_aug, const double *B_aug,
-                               const double *Q_aug, const double *R_inv, const double *z0,
+                               const double *Q_aug, const double *R_inv, long rinv_stride, const double *z0,
                                const double *QT, double *J, double jitter, int max_tries, long *retries)
 {
     if (d < 1 || d > HOP_MAXD || m < 1 || m > HOP_MAXD) return HOP_ERR_ARG;
-    return propagator_all_Jt_f64(T_use, d, m, A_aug, B_aug, Q_aug, R_inv, z0, QT, J, jitter, max_tries, retries);
+    if (rinv_stride != 0 && rinv_stride != (long)m * m) return HOP_ERR_ARG;
+    return propagator_all_Jt_f64(T_use, d, m, A_aug, B_aug, Q_aug, R_inv, rinv_stride, z0, QT, J, jitter, max_tries, retries);
 }
 int hopo_propagator_all_Jt_f80(int T_use, int d, int m, const double *A_aug, const double *B_aug,
-                               const double *Q_aug, const double *R_inv, const double *z0,
+                               const double *Q_aug, const double *R_inv, long rinv_stride, const double *z0,
                                const double *QT, double *J, double jitter, int max_tries, long *retries)
 {
     if (d < 1 || d > HOP_MAXD || m < 1 || m > HOP_MAXD) return HOP_ERR_ARG;
-    return propagator_all_Jt_f80(T_use, d, m, A_aug, B_aug, Q_aug, R_inv, z0, QT, J, jitter, max_tries, retries);
+    if (rinv_stride != 0 && rinv_stride != (long)m * m) return HOP_ERR_ARG;
+    return propagator_all_Jt_f80(T_use, d, m, A_aug, B_aug, Q_aug, R_inv, rinv_stride, z0, QT, J, jitter, max_tries, retries);
 }
 
 /* solver.py:522,590.  np.argmin returns the first minimum and treats NaN as the minimum. */
@@ -410,7 +419,7 @@ int hopo_select_fused(int sys, const double *p, int n, int m, int N, int T_min, 
                       double *J, int *T_star)
 {
     const int d = n + 1;
-    if (T_max > N || T_min < 1 || T_min > T_max) return HOP_ERR_ARG;
+    if (!dims_ok(n, m) || T_max > N || T_min < 1 || T_min > T_max) return HOP_ERR_ARG;
     size_t tot = (size_t)N * (3 * d * d + d * m) + (size_t)N * n;
     double *buf = (double *)malloc(sizeof(double) * tot);
     if (!buf) return HOP_ERR_ALLOC;
@@ -425,8 +434,8 @@ int hopo_select_fused(int sys, const double *p, int n, int m, int N, int T_min, 
         hopo_build_terminal(n, N, X, xg, Qf, wrap_mask, 1e-12, QT);
         for (int i = 0; i < d; ++i) z0[i] = 0.0;
         z0[d - 1] = 1.0; /* augmented.py:59 */
-        rc = use_f80 ? propagator_all_Jt_f80(T_max, d, m, A_aug, B_aug, Q_aug, R_inv, z0, QT, J, HOP_JITTER, HOP_TRIES, NULL)
-                     : propagator_all_Jt_f64(T_max, d, m, A_aug, B_aug, Q_aug, R_inv, z0, QT, J, HOP_JITTER, HOP_TRIES, NULL);
+        rc = use_f80 ? propagator_all_Jt_f80(T_max, d, m, A_aug, B_aug, Q_aug, R_inv, 0, z0, QT, J, HOP_JITTER, HOP_TRIES, NULL)
+                     : propagator_all_Jt_f64(T_max, d, m, A_aug, B_aug, Q_aug, R_inv, 0, z0, QT, J, HOP_JITTER, HOP_TRIES, NULL);
     }
     if (!rc) *T_star = hopo_argmin_window(J, T_min, T_max);
     free(buf);
@@ -473,6 +482,7 @@ int hopo_backward_pass(int n, int m, const double *A, const double *B, const dou
                        double *k_out, double *K_out, int *ok)
 {
     *ok = 0;
+    if (!dims_ok(n, m)) return HOP_ERR_ARG;
     if (T_star <= 0) return HOP_OK;
     double e[HOP_MAXN], du[HOP_MAXM], Vx[HOP_MAXN], Vxx[HOP_MAXN * HOP_MAXN];
     for (int i = 0; i < n; ++i) e[i] = X[(size_t)T_star * n + i] - xg[i];
@@ -592,6 +602,7 @@ int hopo_bruteforce_all_Jt(int n, int m, const double *A, const double *B, const
                            const double *Qf, double w, int T_max, double lm_lambda, unsigned wrap_mask,
                            double *J)
 {
+    if (!dims_ok(n, m)) return HOP_ERR_ARG;
     for (int T = 1; T <= T_max; ++T) {
         double e[HOP_MAXN], du[HOP_MAXM], Vx[HOP_MAXN], Vxx[HOP_MAXN * HOP_MAXN], V0;
         for (int i = 0; i < n; ++i) e[i] = X[(size_t)T * n + i] - xg[i];
@@ -719,6 +730,7 @@ done:
 typedef struct {
     int kind, lo, hi;
     int sys, N, T_min, T_max, central, T_use, d, m, use_f80;
+    long rinv_stride;
     const double *A, *B, *X, *a_resid;
     unsigned wrap_mask;
     const double *p, *x0, *U, *xg, *u_ref, *Q, *R, *Qf, *w;
@@ -751,7 +763,8 @@ static void *hopo_worker(void *arg)
             const size_t dd = (size_t)j->d * j->d, dm = (size_t)j->d * j->m;
             j->status[b] = propagator_all_Jt_f64(j->T_use, j->d, j->m, j->A_aug + (size_t)b * j->N * dd,
                                                  j->B_aug + (size_t)b * j->N * dm, j->Q_aug + (size_t)b * j->N * dd,
-                                                 j->R_inv + (size_t)b * j->m * j->m, j->z0 + (size_t)b * j->d,
+                                                 j->R_inv + (size_t)b * (j->rinv_stride ? j->N : 1) * j->m * j->m,
+                                                 j->rinv_stride, j->z0 + (size_t)b * j->d,
                                                  j->QT + (size_t)b * j->N * dd, j->J + (size_t)b * j->T_use,
                                                  HOP_JITTER, HOP_TRIES, NULL);
         } else {
@@ -817,7 +830,7 @@ int hopo_select_fused_batch(int nthreads, int Bsz, int n, int m, int N, int T_mi
                             const double *Qf, const double *w, unsigned wrap_mask, int use_f80, double *J,
                             int *T_star, int *status)
 {
-    if (n < 1 || n + 1 > HOP_MAXD || m < 1 || m > HOP_MAXM) return HOP_ERR_ARG;
+    if (!dims_ok(n, m)) return HOP_ERR_ARG;
     hopo_job j; memset(&j, 0, sizeof j);
     j.kind = 3; j.d = n; j.m = m; j.N = N; j.T_min = T_min; j.T_max = T_max; j.A = A; j.B = B; j.a_resid = a_resid;
     j.X = X; j.U = U; j.xg = xg; j.u_ref = u_ref; j.Q = Q; j.R = R; j.Qf = Qf; j.w = w; j.wrap_mask = wrap_mask;
@@ -826,13 +839,14 @@ int hopo_select_fused_batch(int nthreads, int Bsz, int n, int m, int N, int T_mi
 }
 
 int hopo_propagator_batch(int nthreads, int Bsz, int N, int T_use, int d, int m, const double *A_aug,
-                          const double *B_aug, const double *Q_aug, const double *R_inv, const double *z0,
-                          const double *QT, double *J, int *status)
+                          const double *B_aug, const double *Q_aug, const double *R_inv, long rinv_stride,
+                          const double *z0, const double *QT, double *J, int *status)
 {
     if (d < 1 || d > HOP_MAXD || m < 1 || m > HOP_MAXD || T_use > N) return HOP_ERR_ARG;
+    if (rinv_stride != 0 && rinv_stride != (long)m * m) return HOP_ERR_ARG;
     hopo_job j; memset(&j, 0, sizeof j);
     j.kind = 1; j.N = N; j.T_use = T_use; j.d = d; j.m = m; j.A_aug = A_aug; j.B_aug = B_aug; j.Q_aug = Q_aug;
-    j.R_inv = R_inv; j.z0 = z0; j.QT = QT; j.J = J; j.status = status;
+    j.R_inv = R_inv; j.rinv_stride = rinv_stride; j.z0 = z0; j.QT = QT; j.J = J; j.status = status;
     return hopo_fan_out(nthreads, Bsz, &j);
 }
 

@@ -41,7 +41,9 @@ void hopo_wrap_error(int n, double *e, unsigned wrap_mask);
 int hopo_sys_dims(int sys, int *n, int *m);
 void hopo_dynamics(int sys, const double *p, const double *x, const double *u, double *xn);
 
-/* ---- solver.py primitives ---- */
+/* ---- solver.py primitives ----
+ * Every entry point below that takes the state / control dimensions n, m (not a system id) needs
+ * 1 <= n <= 15 and 1 <= m <= 16 and returns HOP_ERR_ARG otherwise (hopo_cost_timeopt_true: NaN). */
 void hopo_rollout(int sys, const double *p, int N, const double *x0, const double *U, double *X,
                   double max_state_norm);
 double hopo_cost_timeopt_true(int n, int m, const double *X, const double *U, const double *xg,
@@ -71,15 +73,17 @@ int hopo_build_augmented(int n, int m, int N, const double *A, const double *B, 
                          const double *X, const double *U, const double *xg, const double *u_ref,
                          const double *Q, const double *R, double w, unsigned wrap_mask, double q_reg,
                          double rho_reg, double *A_aug, double *B_aug, double *Q_aug, double *R_inv);
-void hopo_build_terminal(int n, int N, const double *X, const double *xg, const double *Qf,
-                         unsigned wrap_mask, double rho_reg, double *QT);
+int hopo_build_terminal(int n, int N, const double *X, const double *xg, const double *Qf,
+                        unsigned wrap_mask, double rho_reg, double *QT);
 
-/* ---- horizon_selection.py ---- */
+/* ---- horizon_selection.py ----
+ * R_inv is [m][m] (rinv_stride = 0: the R_inv_cached argument) or [N][m][m] (rinv_stride = m*m: chol_inv(R_list[k])
+ * per step, horizon_selection.py:60-61); hopo_propagator_batch: [B][m][m] or [B][N][m][m]. */
 int hopo_propagator_all_Jt_f64(int T_use, int d, int m, const double *A_aug, const double *B_aug,
-                               const double *Q_aug, const double *R_inv, const double *z0,
+                               const double *Q_aug, const double *R_inv, long rinv_stride, const double *z0,
                                const double *QT, double *J, double jitter, int max_tries, long *retries);
 int hopo_propagator_all_Jt_f80(int T_use, int d, int m, const double *A_aug, const double *B_aug,
-                               const double *Q_aug, const double *R_inv, const double *z0,
+                               const double *Q_aug, const double *R_inv, long rinv_stride, const double *z0,
                                const double *QT, double *J, double jitter, int max_tries, long *retries);
 /* solver.py:522,590: int(np.argmin(J[T_min-1:T_max]) + T_min)  (first minimum; NaN wins) */
 int hopo_argmin_window(const double *J, int T_min, int T_max);
@@ -114,8 +118,8 @@ int hopo_select_fused_batch(int nthreads, int Bsz, int n, int m, int N, int T_mi
                             const double *Qf, const double *w, unsigned wrap_mask, int use_f80, double *J,
                             int *T_star, int *status);
 int hopo_propagator_batch(int nthreads, int Bsz, int N, int T_use, int d, int m, const double *A_aug,
-                          const double *B_aug, const double *Q_aug, const double *R_inv, const double *z0,
-                          const double *QT, double *J, int *status);
+                          const double *B_aug, const double *Q_aug, const double *R_inv, long rinv_stride,
+                          const double *z0, const double *QT, double *J, int *status);
 
 /* solver.py:449-765  ilqr_timeopt(method="propagator") */
 typedef struct {

@@ -244,3 +244,54 @@ def test_oracle_full_solves_match_the_reference_on_sampled_initial_states(name):
         assert (same & well).sum() == well.sum(), np.nonzero(well & ~same)[0]
         assert max(relJ) <= 1e-9
         assert (o["T_star"][well] == g[name + "_T_star"][well]).all()
+
+
+@pytest.mark.parametrize("f80", [False, True])
+def test_per_step_rinv_constant_over_k_is_bit_identical_to_one_rinv(f80):
+    """R_inv [N, m, m] (a different R^-1 per step, horizon_selection.py:60-61) reloads R^-1 at every step; with the same R^-1
+    at every step it must give the bits of the single-R^-1 path, in both precisions and through the batched entry."""
+    from _common import s2_batch
+    d, m, N, B = 5, 3, 12, 3
+    A, Bm, Q, R, z0, w, QT = s2_batch(range(B), d, m, N)
+    Rinv = np.stack([O.chol_inv(r) for r in R])
+    for b in range(B):
+        J1 = O.propagator_all_Jt(A[b], Bm[b], Q[b], Rinv[b], z0[b], QT[b], f80=f80)
+        Jk = O.propagator_all_Jt(A[b], Bm[b], Q[b], np.repeat(Rinv[b][None], N, 0), z0[b], QT[b], f80=f80)
+        assert np.isfinite(J1).all() and np.array_equal(J1, Jk)
+    if not f80:
+        Jb, st = O.propagator_batch(A, Bm, Q, np.repeat(Rinv[:, None], N, 1), z0, QT, nthreads=2)
+        Jo, sto = O.propagator_batch(A, Bm, Q, Rinv, z0, QT)
+        assert not st.any() and not sto.any() and np.array_equal(Jb, Jo)
+    with pytest.raises(ValueError):                       # a per-step R^-1 must cover every step
+        O.propagator_all_Jt(A[0], Bm[0], Q[0], np.repeat(Rinv[0][None], N - 1, 0), z0[0], QT[0])
+
+
+@pytest.mark.parametrize("m", [9, 16])
+def test_select_fused_takes_control_dimensions_up_to_16(m):
+    from _common import fused_batch
+    n, N = 15, 6
+    g = fused_batch(3, 2, n, m, N)
+    for b in range(2):
+        J, T = O.select_fused(g["A"][b], g["Bm"][b], g["X"][b], g["U"], g["xg"][b], g["u_ref"], g["Q"], g["R"], g["alpha"],
+                              g["w"][b], 2, N - 1, g["wrap_idx"], a_resid=g["a"][b])
+        assert np.isfinite(J).all() and 2 <= T <= N - 1 and T == np.argmin(J[1:N - 1]) + 2
+    J, T, st = O.select_fused_batch(g["A"], g["Bm"], g["X"], g["U"], g["xg"], g["u_ref"], g["Q"], g["R"], g["alpha"], g["w"],
+                                    2, N - 1, g["wrap_idx"], a_resid=g["a"])
+    assert not st.any() and np.isfinite(J).all()
+
+
+def test_select_fused_rejects_dimensions_beyond_its_arrays():
+    """m > 16 or n > 15 is an argument error, not a write past the oracle's stack arrays."""
+    from _common import fused_batch
+    for n, m in ((15, 17), (16, 4)):
+        g = fused_batch(4, 1, n, m, 4)
+        with pytest.raises(RuntimeError, match="error code 4"):
+            O.select_fused(g["A"][0], g["Bm"][0], g["X"][0], g["U"], g["xg"][0], g["u_ref"], g["Q"], g["R"], g["alpha"],
+                           g["w"][0], 1, 4, g["wrap_idx"])
+        with pytest.raises(RuntimeError, match="error code 4"):
+            O.build_augmented(g["A"][0], g["Bm"][0], None, g["X"][0], g["U"], g["xg"][0], g["u_ref"], g["Q"], g["R"],
+                              g["w"][0])
+        with pytest.raises(RuntimeError, match="error code 4"):
+            O.backward_pass(g["A"][0], g["Bm"][0], g["X"][0], g["U"], g["xg"][0], g["u_ref"], g["Q"], g["R"], g["alpha"], 3)
+        assert np.isnan(O.cost_timeopt_true(g["X"][0], g["U"], g["xg"][0], g["u_ref"], g["Q"], g["R"], g["alpha"],
+                                            g["w"][0], 3))
