@@ -243,11 +243,11 @@ int hop_ilqr_timeopt_f64(int B, int sys, const double *params_host, int N, int T
                          double *J_hist, int *T_hist, int *n_hist, double *J_curve, int *T_star, int *status,
                          int *iters_run_host, double *timers_host, void *stream);
 
-/* Test hook: selects the quadrotor forward-difference kernel (0 = thread per step [default], 1 = lane per column,
- * 2 = the generic kernel); returns the previous value.  All three produce identical bits (tests/test_gpu_parity.py). */
+/* Test hook: selects the quadrotor finite-difference kernel (0 = thread per step [default], 2 = the generic kernel; any
+ * other value is ignored); returns the previous value.  Both produce identical bits (tests/test_gpu_parity.py). */
 int hop_test_set_linearize_variant(int variant);
 /* Test hook: smallest batch hop_select_f64 routes to the thread-per-problem kernel (d <= 5).  -1 = the built-in defaults
- * (d <= 4: every batch; d = 5: B >= 16384), >= 0 = that threshold for every d (0 = always; also $HOP_TPP_MIN_BATCH),
+ * (d <= 4: every batch; d = 5: B >= 16384), >= 0 = that threshold for every d (0 = always),
  * < -1 = query only.  Below the threshold the lane-group kernel runs; the two produce identical bits.  Returns the
  * previous value. */
 long hop_test_set_tpp_min_batch(long min_batch);
@@ -259,9 +259,9 @@ int hop_test_set_generic_pre(int on);
  * Gauss-Jordan sweep of a diagonal matrix computes anyway), 0 = by the sweep like any other block; identical bits.  Returns the
  * previous value. */
 int hop_test_set_generic_diag(int on);
-/* Test hook: fused selection kernel of the small systems (n <= 4).  0 [default] = by batch size: up to $HOP_WSP_MAX_BATCH = 592
- * instances one problem per CTA as a warp-specialised pipeline (stage / prefix / query warps, one matrix element per lane), up to
- * $HOP_EPL_MAX_BATCH = 1024 one warp per problem (one element per lane), a lane group per problem above; 1 = lane group,
+/* Test hook: fused selection kernel of the small systems (n <= 4).  0 [default] = by batch size: up to 592 instances one
+ * problem per CTA as a warp-specialised pipeline (stage / prefix / query warps, one matrix element per lane), up to 1024
+ * one warp per problem (one element per lane), a lane group per problem above; 1 = lane group,
  * 2 = pipeline, 3 = one warp per problem.  All three perform the same IEEE operations per element: identical bits.  Returns the
  * previous value. */
 int hop_test_set_fused_small_variant(int variant);

@@ -1,6 +1,5 @@
 // hop_cabi.cu -- extern "C" surface of libhop_b200.so (see include/hop_b200.h for the contract).
 #include <cstring>
-#include <cstdlib>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -535,7 +534,7 @@ long hop_test_set_tpp_min_batch(long min_batch) { return hop::tpp_min_batch(min_
 
 int hop_test_set_linearize_variant(int variant) {
     const int old = g_linearize_variant;
-    if (variant >= 0 && variant <= 2) g_linearize_variant = variant;
+    if (variant == 0 || variant == 2) g_linearize_variant = variant;
     return old;
 }
 
@@ -573,33 +572,21 @@ int hop_probe_fp64_tflops(int iters, double* tflops_out, double* ms_out) {
 // and the inputs of chunk c+1 arrive, so only the first upload and the last download are exposed.  It also bounds
 // the linearisation workspace (A, B: 1.7 KB per instance and step) to two chunks instead of the whole batch.
 // Measured (profiles/r2_experiments.txt): one step = 44.3 ms against 43.7 ms of kernels (selection 39.4 + linearisation 3.6 +
-// rollout 0.74).  HOP_HOST_PRIO_PREP=1 moves the HBM-bound rollout / linearisation of every chunk to a HIGH-PRIORITY
-// stream so that they could run under the FP64-bound selection of the previous chunk; on B200 that bought nothing
-// (44.7 ms with 8 chunks, 44.5 ms with 4: the selection kernel holds every SM's register file, a freed slot goes to a
-// linearisation block and the displaced selection work returns later), so it stays an opt-in A/B switch.
+// rollout 0.74).  Running the rollout / linearisation of every chunk on a high-priority stream, under the selection of the
+// previous chunk, bought nothing (B200: 44.52 against 44.34 ms per step, profiles/r2_experiments.txt item 1).
 namespace {
-constexpr int kHostChunksCap = 16;
 struct HostCtx {
     std::mutex mu;
     cudaStream_t stream[2] = {nullptr, nullptr};
-    cudaStream_t pre = nullptr;                       // high priority: rollout + linearisation
     cudaEvent_t consts_ready = nullptr;
-    cudaEvent_t up[kHostChunksCap] = {}, prep[kHostChunksCap] = {}, sel[kHostChunksCap] = {};
     void* buf = nullptr;
     size_t cap = 0;
     int device = -1;
     void reset() {
         if (buf) cudaFree(buf);
         for (auto& st : stream) { if (st) cudaStreamDestroy(st); st = nullptr; }
-        if (pre) cudaStreamDestroy(pre);
         if (consts_ready) cudaEventDestroy(consts_ready);
-        for (int i = 0; i < kHostChunksCap; ++i) {
-            if (up[i]) cudaEventDestroy(up[i]);
-            if (prep[i]) cudaEventDestroy(prep[i]);
-            if (sel[i]) cudaEventDestroy(sel[i]);
-            up[i] = prep[i] = sel[i] = nullptr;
-        }
-        buf = nullptr; cap = 0; pre = nullptr; consts_ready = nullptr;
+        buf = nullptr; cap = 0; consts_ready = nullptr;
     }
 };
 HostCtx g_host;
@@ -625,22 +612,11 @@ int hop_select_from_x0_host_f64(int B, int sys, const double* params_host, int N
     }
     for (auto& st : g_host.stream)
         if (!st) { if (int rc = report_cuda(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking), "cudaStreamCreate")) return rc; }
-    if (!g_host.pre) {
-        int lo = 0, hi = 0;                                                      // (numerically lower = higher priority)
-        cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        if (int rc = report_cuda(cudaStreamCreateWithPriority(&g_host.pre, cudaStreamNonBlocking, hi), "cudaStreamCreateWithPriority")) return rc;
-    }
     if (!g_host.consts_ready) {
         if (int rc = report_cuda(cudaEventCreateWithFlags(&g_host.consts_ready, cudaEventDisableTiming), "cudaEventCreate")) return rc;
-        for (int i = 0; i < kHostChunksCap; ++i)
-            for (cudaEvent_t* e : {&g_host.up[i], &g_host.prep[i], &g_host.sel[i]})
-                if (int rc = report_cuda(cudaEventCreateWithFlags(e, cudaEventDisableTiming), "cudaEventCreate")) return rc;
     }
-    static const int chunks_max = getenv("HOP_HOST_CHUNKS") ? atoi(getenv("HOP_HOST_CHUNKS")) : kHostChunksMax;   // A/B switch
     int chunks = (B + kHostChunkMin - 1) / kHostChunkMin;
-    chunks = chunks < 1 ? 1 : (chunks > chunks_max ? chunks_max : chunks);
-    if (chunks < 1) chunks = 1;
-    if (chunks > kHostChunksCap) chunks = kHostChunksCap;
+    chunks = chunks < 1 ? 1 : (chunks > kHostChunksMax ? kHostChunksMax : chunks);
     const int per = (((B + chunks - 1) / chunks) + 3) & ~3;       // whole CTAs of the selection kernel
     const int lanes = chunks > 1 ? 2 : 1;                         // workspaces (= streams) in use
     const bool shared_U = (u_batch_stride == 0);
@@ -681,14 +657,11 @@ int hop_select_from_x0_host_f64(int B, int sys, const double* params_host, int N
     if (shared_U) copy(d_U, U, sizeof(double) * nU, cudaMemcpyHostToDevice, s0, "H2D U");
     if (rc == 0) rc = report_cuda(cudaEventRecord(g_host.consts_ready, s0), "cudaEventRecord");
     if (rc == 0 && lanes > 1) rc = report_cuda(cudaStreamWaitEvent(g_host.stream[1], g_host.consts_ready, 0), "cudaStreamWaitEvent");
-    if (rc == 0) rc = report_cuda(cudaStreamWaitEvent(g_host.pre, g_host.consts_ready, 0), "cudaStreamWaitEvent");
-    static const bool serial_prep = !(getenv("HOP_HOST_PRIO_PREP") && atoi(getenv("HOP_HOST_PRIO_PREP")) != 0);   // A/B switch (default: serial)
     for (int c = 0; c < chunks && rc == 0; ++c) {
         const int b0 = c * per, cb = (B - b0) < per ? (B - b0) : per;
         if (cb <= 0) break;
         const int lane = c % lanes;
         cudaStream_t st = g_host.stream[lane];
-        cudaStream_t sp = serial_prep ? st : g_host.pre;
         const size_t o = (size_t)b0;
         copy(d_x0 + o * n, x0 + o * n, sizeof(double) * (size_t)cb * n, cudaMemcpyHostToDevice, st, "H2D x0");
         copy(d_xg + o * n, xg + o * n, sizeof(double) * (size_t)cb * n, cudaMemcpyHostToDevice, st, "H2D xg");
@@ -704,34 +677,23 @@ int hop_select_from_x0_host_f64(int B, int sys, const double* params_host, int N
         double* Xc = (double*)wsl;
         double* Ac = (double*)(wsl + align256(sizeof(double) * (size_t)per * (N + 1) * n));
         double* Bc = (double*)((char*)Ac + align256(sizeof(double) * (size_t)per * N * n * n));
-        if (!serial_prep) {
-            if ((rc = report_cuda(cudaEventRecord(g_host.up[c], st), "cudaEventRecord"))) break;
-            if ((rc = report_cuda(cudaStreamWaitEvent(sp, g_host.up[c], 0), "cudaStreamWaitEvent"))) break;
-            if (c >= lanes && (rc = report_cuda(cudaStreamWaitEvent(sp, g_host.sel[c - lanes], 0), "cudaStreamWaitEvent"))) break;   // workspace re-use
-        }
-        if ((rc = dispatch_rollout(cb, sys, params_host, N, d_x0 + o * n, dU, u_batch_stride, 1e6, Xc, sp))) break;         // solver.py:42
+        if ((rc = dispatch_rollout(cb, sys, params_host, N, d_x0 + o * n, dU, u_batch_stride, 1e6, Xc, st))) break;         // solver.py:42
         // X comes from the rollout above, so F(X_k, U_k) = X[k+1] bit for bit: the linearisation may read f0 from it
         if ((rc = dispatch_linearize(cb, sys, params_host, N, Xc, dU, u_batch_stride, central, 1e-5, 1e-5, 1e-6, 1e-6, 1, nullptr,
-                                     Ac, Bc, sp))) break;                                                                  // linearization.py:177,216
-        if (!serial_prep) {
-            if ((rc = report_cuda(cudaEventRecord(g_host.prep[c], sp), "cudaEventRecord"))) break;
-            if ((rc = report_cuda(cudaStreamWaitEvent(st, g_host.prep[c], 0), "cudaStreamWaitEvent"))) break;
-        }
+                                     Ac, Bc, st))) break;                                                                  // linearization.py:177,216
         // a_resid = NULL: on a trajectory produced by the rollout above F(X_k,U_k) - X_{k+1} is exactly 0
         rc = hop_select_fused_f64(cb, N, n, m, T_min, T_max, Ac, Bc, nullptr, Xc, dU, u_batch_stride, d_xg + o * n, d_w + o, d_uref,
                                   d_Q, d_R, d_Qf, wrap_mask, 1e-9, 1e-12, mode, d_J + o * T_max, d_T + o, d_Js + o, d_st + o, st);
         if (rc) break;
-        if ((rc = report_cuda(cudaEventRecord(g_host.sel[c], st), "cudaEventRecord"))) break;
         if (J_out) copy(J_out + o * T_max, d_J + o * T_max, sizeof(double) * (size_t)cb * T_max, cudaMemcpyDeviceToHost, st, "D2H J");
         copy(Tstar_out + o, d_T + o, sizeof(int) * (size_t)cb, cudaMemcpyDeviceToHost, st, "D2H T*");
         if (Jstar_out) copy(Jstar_out + o, d_Js + o, sizeof(double) * (size_t)cb, cudaMemcpyDeviceToHost, st, "D2H J*");
         if (status) copy(status + o, d_st + o, sizeof(int) * (size_t)cb, cudaMemcpyDeviceToHost, st, "D2H status");
     }
-    cudaError_t ep = cudaStreamSynchronize(g_host.pre);
     cudaError_t e0 = cudaStreamSynchronize(g_host.stream[0]);
     cudaError_t e1 = lanes > 1 ? cudaStreamSynchronize(g_host.stream[1]) : cudaSuccess;
     if (rc) return rc;
-    return report_cuda(e0 != cudaSuccess ? e0 : (e1 != cudaSuccess ? e1 : ep), "hop_select_from_x0_host_f64");
+    return report_cuda(e0 != cudaSuccess ? e0 : e1, "hop_select_from_x0_host_f64");
 }
 
 }  // extern "C"

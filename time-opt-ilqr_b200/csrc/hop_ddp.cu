@@ -9,7 +9,6 @@
 // Every kernel takes the per-instance `done` word and skips finished instances, so a batch whose
 // members stop at different iterations needs no host-side control flow.
 #include "hop_common.cuh"
-#include <cstdlib>
 
 #include "hop_ddp_core.cuh"
 #include "hop_ddp_mma.cuh"
@@ -84,8 +83,8 @@ __global__ void k_backward(int B, int N, const double* A, const double* Bm, cons
 // backward-pass kernel: 0 [default] = the tensor-pipe kernel (backward_pass_mma) for n > 8 unless the caller asks for the
 // reference's summation order (HOP_MODE_EXACT solves, the stand-alone entry point), else the warp kernel; 1 = one thread per
 // problem; 2 = one warp per problem, ordered sums (1 and 2: identical bits); 3 = tensor-pipe kernel wherever it is instantiated.
-// $HOP_BW_VARIANT / hop_test_set_backward_variant ($HOP_BW_THREAD=1 is the old spelling of variant 1)
-int g_backward_variant = getenv("HOP_BW_VARIANT") ? atoi(getenv("HOP_BW_VARIANT")) : (getenv("HOP_BW_THREAD") && atoi(getenv("HOP_BW_THREAD")) ? 1 : 0);
+// Set by hop_test_set_backward_variant.
+int g_backward_variant = 0;
 
 // one warp per problem (backward_pass_warp), kBwWarps problems per CTA
 constexpr int kBwWarps = 4;
@@ -247,9 +246,9 @@ __global__ void __launch_bounds__(kLsRoles * 32) k_linesearch_par(int B, DynPara
     for (size_t i = role; i < (size_t)N * m; i += kLsRoles) Unb[i] = Ub[i];
     if (role == 0) { Jn[b] = J_old; acc[b] = 0; }
 }
-// line-search kernel: 0 step sizes side by side (default), 1 one thread per problem trying them in turn (test / A-B hook;
+// line-search kernel: 0 step sizes side by side (default), 1 one thread per problem trying them in turn (test hook;
 // identical bits)
-int g_linesearch_variant = getenv("HOP_LS_SERIAL") ? atoi(getenv("HOP_LS_SERIAL")) : 0;
+int g_linesearch_variant = 0;
 template <int SYS>
 static int launch_linesearch(int B, const DynParams2& prm, int N, const double* X, const double* U, const DdpConst& c, const int* T,
                              const double* kl, const double* Kl, const int* ok, const int* done, double* Xn, double* Un,
@@ -257,8 +256,8 @@ static int launch_linesearch(int B, const DynParams2& prm, int N, const double* 
     const int threads = 64;
     // Six threads per instance only pay while they fit next to each other: measured on B200, forward phase of a 12-iteration
     // solve: Segway B = 25 7.6 -> 2.5 ms, Cartpole B = 4096 67.5 -> 16.1 ms, Quadrotor B = 16384 22.1 -> 28.3 ms (130
-    // registers: the machine holds ~75k such threads, 16384 x 6 no longer fit in one wave).  $HOP_LS_PAR_MAX_BATCH overrides.
-    static const long par_max = getenv("HOP_LS_PAR_MAX_BATCH") ? atol(getenv("HOP_LS_PAR_MAX_BATCH")) : 8192;
+    // registers: the machine holds ~75k such threads, 16384 x 6 no longer fit in one wave).
+    constexpr long par_max = 8192;
     if (g_linesearch_variant != 0 || B > par_max) {
         k_linesearch<SYS><<<(B + threads - 1) / threads, threads, 0, st>>>(B, prm, N, X, U, c, T, kl, Kl, ok, done, Xn, Un, Jn, acc);
         return check_launch("k_linesearch");

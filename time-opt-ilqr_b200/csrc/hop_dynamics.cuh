@@ -66,8 +66,8 @@ HOP_DEVICE void dynamics<3>(const double* p, const double* x, const double* u, d
     xn[0] = n0; xn[1] = n1; xn[2] = n2; xn[3] = n3;
 }
 // systems.py:170-210 (rotm :145-156, Tmat :158-163, guards :175-191), split so that the finite-difference
-// kernel can share the trigonometry of the unperturbed angles between the lanes of a (problem, step) group;
-// dynamics<2> below and k_linearize_quad evaluate exactly the same operation sequence.
+// kernel can share the trigonometry of the unperturbed angles between the 16 perturbed evaluations of a (problem, step);
+// dynamics<2> below and k_linearize_quad_row evaluate exactly the same operation sequence.
 struct QuadTrig { double sph, cph, sth, cth, tth, sps, cps; };
 
 // the guards that do not need trigonometry (systems.py:175-183,188-191)

@@ -5,7 +5,6 @@
 // load-balances warps across the 148 SMs.  Dynamic shared memory = per-group slab (Geo::SLAB
 // doubles) [+ the CTA-wide case constants for the fused form].
 #include <cstdint>
-#include <cstdlib>
 
 #include "hop_common.cuh"
 #include "hop_select_body.cuh"
@@ -142,9 +141,7 @@ __global__ void __launch_bounds__(kMmaWarps * 32, 3) k_select_generic_pipe(const
 }
 // ---- pre-inverted input blocks: E_k = chol_inv(Q_k), X_t = chol_inv(QT_t) for every (problem, step) in parallel --------
 constexpr int kPreWarps = 4;
-#ifndef PRE_MINB
-#define PRE_MINB 4   // CTAs per SM the pre-pass is register-bounded for (2 -> 174 registers, 4 -> 128)
-#endif
+constexpr int PRE_MINB = 4;   // CTAs per SM the pre-pass is register-bounded for (2 -> 174 registers, 4 -> 128)
 // four lanes per matrix, eight matrices per warp; matrix index = 2 (b T_max + k) + {0: Q_aug, 1: QT}
 template <int D>
 __global__ void __launch_bounds__(kPreWarps * 32, PRE_MINB) k_preinvert(const SelectArgs p, double* E, double* X, int* bad) {
@@ -198,9 +195,9 @@ void stream_free(void* ptr, cudaStream_t st) {
 // 1: always, 0: never (sweep B inside the sequential kernel), -1 [default]: for small batches only.  Measured on B200
 // (S2, d = 13, N = 128): B = 8: 0.95 -> 0.76 ms (one sweep latency per step instead of two); B = 65 536: 63.3 -> 68.2 ms
 // (sequential kernel 63.3 -> 46.5 ms, but the pre-pass moves 45 GB and costs 19.8 ms): it pays where latency matters.
-int g_generic_pre = getenv("HOP_GENERIC_PRE") ? atoi(getenv("HOP_GENERIC_PRE")) : -1;
-// 1: diagonal input blocks go through the Gauss-Jordan sweep like any other block (A/B switch + test hook); 0 [default]: element-wise
-int g_generic_nodiag = getenv("HOP_GENERIC_NODIAG") ? atoi(getenv("HOP_GENERIC_NODIAG")) : 0;
+int g_generic_pre = -1;
+// 1: diagonal input blocks go through the Gauss-Jordan sweep like any other block (test hook); 0 [default]: element-wise
+int g_generic_nodiag = 0;
 constexpr int kGenericPreMaxBatch = 1024;
 
 template <int D, int M>
@@ -250,33 +247,13 @@ static int launch_generic_pipe(const SelectArgs& p, cudaStream_t st) {
     return rc_all;
 }
 
-// MINB = CTAs per SM the register allocation is bounded for (2 -> 255 regs, 3 -> 168, 4 -> 128).
-static int mma_min_blocks() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("HOP_MMA_MINBLOCKS");
-        v = e ? atoi(e) : 3;
-        if (v < 2 || v > 4) v = 3;
-    }
-    return v;
-}
-template <int D, int M, int MODE, int MINB>
-static int launch_fused_mma_b(const FusedArgs& p, cudaStream_t st) {
-    const size_t smem = sizeof(double) * ((size_t)kMmaWarps * mma::kWarpScratch + mma::PipeConst<D, M>::SIZE);
-    const int grid = (p.B + kMmaWarps - 1) / kMmaWarps;
-    k_select_fused_mma<D, M, MODE, MINB><<<grid, kMmaWarps * 32, smem, st>>>(p);
-    return check_launch("k_select_fused_mma");
-}
+// MINB = CTAs per SM the register allocation is bounded for (2 -> 255 regs, 3 [the only one instantiated] -> 168, 4 -> 128).
 template <int D, int M, int MODE>
 static int launch_fused_mma(const FusedArgs& p, cudaStream_t st) {
-    if constexpr (MODE == 5) {   // the occupancy A/B ($HOP_MMA_MINBLOCKS) exists for the default schedule only (compile time)
-        switch (mma_min_blocks()) {
-            case 2: return launch_fused_mma_b<D, M, MODE, 2>(p, st);
-            case 4: return launch_fused_mma_b<D, M, MODE, 4>(p, st);
-            default: break;
-        }
-    }
-    return launch_fused_mma_b<D, M, MODE, 3>(p, st);
+    const size_t smem = sizeof(double) * ((size_t)kMmaWarps * mma::kWarpScratch + mma::PipeConst<D, M>::SIZE);
+    const int grid = (p.B + kMmaWarps - 1) / kMmaWarps;
+    k_select_fused_mma<D, M, MODE, 3><<<grid, kMmaWarps * 32, smem, st>>>(p);
+    return check_launch("k_select_fused_mma");
 }
 
 

@@ -26,7 +26,7 @@ struct SelectArgs {
     // E_pre[b][k] = chol_inv(Q_aug[b][k]), X_pre[b][k] = chol_inv(QT[b][k]), pre_bad[b] != 0 => some inversion needs the ladder
     const double *E_pre, *X_pre;
     const int* pre_bad;
-    // test hook (hop_test_set_generic_diag / $HOP_GENERIC_NODIAG): non-zero => the pipelined LQR-boundary kernel inverts DIAGONAL
+    // test hook (hop_test_set_generic_diag): non-zero => the pipelined LQR-boundary kernel inverts DIAGONAL
     // input blocks by the Gauss-Jordan sweep like any other block instead of element-wise (identical bits either way)
     int no_diag_fastpath;
 };

@@ -1,8 +1,6 @@
 // hop_select_epl.cu -- __global__ wrapper + launcher of the element-per-lane fused selection kernel for small systems
 // (hop_select_epl_body.cuh).  Grid: one warp per problem, kEplWarps warps per CTA (small CTAs spread a small batch
 // over many SMs: these launches are latency bound).  Dynamic shared memory = per-warp LU scratch + the CTA constants.
-#include <cstdlib>
-
 #include "hop_common.cuh"
 #include "hop_select_epl_body.cuh"
 #include "../../include/hop_b200.h"
@@ -80,18 +78,17 @@ static int launch_fused_wsp(const FusedArgs& p, cudaStream_t st) {
 }
 
 // fused selection kernel of the small systems: 0 routing by batch size (default), 1 lane group per problem, 2 warp-specialised
-// pipeline, 3 element per lane, one warp (test / A-B hook; all three give identical bits)
-int g_fused_small_variant = getenv("HOP_FUSED_LANES") ? atoi(getenv("HOP_FUSED_LANES")) : 0;
+// pipeline, 3 element per lane, one warp (test hook; all three give identical bits)
+int g_fused_small_variant = 0;
 
 // A warp per problem only pays while the batch leaves the machine empty (measured on B200, x0 -> T* pipeline, element per
 // lane vs lane group: Segway B = 25 0.86 vs 1.30 ms, Cartpole B = 25 1.42 vs 2.13 ms, DI B = 25 0.28 vs 0.40 ms; at
-// B = 4096 the lane-group kernel, which packs 4-8 problems into a warp, is ahead: 2.15 vs 1.88 ms).  $HOP_EPL_MAX_BATCH overrides.
-// The pipeline spends seven warps on a problem: it pays while the batch leaves most SMs idle ($HOP_WSP_MAX_BATCH, default 4 CTAs
-// per SM; cartpole select phase, pipeline vs one warp per problem, ms: 148 instances 4.29 / 11.8, 296: 5.72 / 11.8, 444: 10.4 / 12.3,
+// B = 4096 the lane-group kernel, which packs 4-8 problems into a warp, is ahead: 2.15 vs 1.88 ms).
+// The pipeline spends seven warps on a problem: it pays while the batch leaves most SMs idle (up to 592 =
+// 4 CTAs per SM; cartpole select phase, pipeline vs one warp per problem, ms: 148 instances 4.29 / 11.8, 296: 5.72 / 11.8, 444: 10.4 / 12.3,
 // 592: 11.1 / 12.3, 1 024 (before the deferred prefix update): 20.7 / 14.3).
+constexpr long max_batch = 1024, wsp_max_batch = 592;
 int dispatch_select_fused_epl(int n, int m, const FusedArgs& p, cudaStream_t st) {
-    static const long max_batch = getenv("HOP_EPL_MAX_BATCH") ? atol(getenv("HOP_EPL_MAX_BATCH")) : 1024;
-    static const long wsp_max_batch = getenv("HOP_WSP_MAX_BATCH") ? atol(getenv("HOP_WSP_MAX_BATCH")) : 592;
     const int v = g_fused_small_variant;
     if (v == 1 || (v == 0 && p.B > max_batch)) return HOP_E_UNSUPPORTED_DIMS;
     const bool wsp = (v == 2) || (v == 0 && p.B <= wsp_max_batch);

@@ -310,17 +310,9 @@ HOP_DEVICE void select_fused_epl_body(const FusedArgs& p, int b, double* scratch
 // 7.56 / 11.8): 2 + 1 + 3 warps 2.68 / 5.94, 1 + 1 + 3: 2.98 / 6.10, 3 + 1 + 3: 2.34 / 4.98 [default], 4 + 1 + 3 and 3 + 1 + 4:
 // 2.70 / 6.03 -- with seven warps the recursion (warp 3) is alone on its SM sub-partition, an eighth warp shares it.
 // ---------------------------------------------------------------------------------------------------------------------
-#ifndef HOP_WSP_STAGE_WARPS
-#define HOP_WSP_STAGE_WARPS 3
-#endif
-#ifndef HOP_WSP_QUERY_WARPS
-#define HOP_WSP_QUERY_WARPS 3
-#endif
-#ifndef HOP_WSP_RING_PER_STAGE
-#define HOP_WSP_RING_PER_STAGE 1
-#endif
-constexpr int kWspStageWarps = HOP_WSP_STAGE_WARPS, kWspQueryWarps = HOP_WSP_QUERY_WARPS, kWspWarps = kWspStageWarps + 1 + kWspQueryWarps;
-constexpr int kWspStageRing = kWspStageWarps * HOP_WSP_RING_PER_STAGE;   // stage -> prefix ring slots
+constexpr int kWspStageWarps = 3, kWspQueryWarps = 3, kWspWarps = kWspStageWarps + 1 + kWspQueryWarps;
+constexpr int kWspRingPerStage = 1;
+constexpr int kWspStageRing = kWspStageWarps * kWspRingPerStage;   // stage -> prefix ring slots
 // named barrier ids (0 is __syncthreads): full / empty per ring slot
 constexpr int kBarStageFull = 1, kBarStageEmpty = kBarStageFull + kWspStageRing;
 constexpr int kBarPrefixFull = kBarStageEmpty + kWspStageRing, kBarPrefixEmpty = kBarPrefixFull + kWspQueryWarps;

@@ -2,7 +2,6 @@
 // (hop_select_tpp_body.cuh).  Grid: one warp per CTA, 32 problems per warp; dynamic shared memory = the warp's
 // double-buffered input stage.
 #include <cstdint>
-#include <cstdlib>
 
 #include "hop_common.cuh"
 #include "hop_select_tpp_body.cuh"
@@ -29,10 +28,9 @@ static int launch_generic_tpp(const SelectArgs& p, cudaStream_t st) {
 // Which batches go to the thread-per-problem kernel (measured on B200, N = 128, profiles/r1h_tpp_vs_lanes.txt): for
 // d <= 4 it is faster than the lane-group kernel at EVERY batch size (B = 32: 0.38 vs 0.55 ms, B = 2^19: 8.8 vs 30.6 ms);
 // for d = 5 its register spills make one step slower (1.0 vs 0.67 ms for a single wave), so it only pays once the batch
-// fills the machine.  -1 = these defaults; >= 0 (test hook or $HOP_TPP_MIN_BATCH) = one threshold for every d.
-static long g_tpp_min_batch = -2;
+// fills the machine.  -1 = these defaults; >= 0 (test hook) = one threshold for every d.
+static long g_tpp_min_batch = -1;
 long tpp_min_batch(long set_to) {   // set_to < -1: query only.  Returns the previous value.
-    if (g_tpp_min_batch == -2) g_tpp_min_batch = getenv("HOP_TPP_MIN_BATCH") ? atol(getenv("HOP_TPP_MIN_BATCH")) : -1;
     const long old = g_tpp_min_batch;
     if (set_to >= -1) g_tpp_min_batch = set_to;
     return old;

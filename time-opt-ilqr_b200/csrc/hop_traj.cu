@@ -4,8 +4,6 @@
 //   k_linearize : linearization.py:216-262 (forward) / :177-211 (central)
 //                 one thread per (problem, step, perturbed coordinate); the n+m threads of a
 //                 (problem, step) pair are adjacent, so each row of A_k / B_k is written coalesced.
-#include <cstdlib>
-
 #include "hop_common.cuh"
 #include "hop_dynamics.cuh"
 #include "../../include/hop_b200.h"
@@ -14,8 +12,8 @@ namespace hop {
 
 struct DynParams { double p[HOP_NPARAMS]; };
 
-// quadrotor forward-difference kernel: 0 thread-per-step (default), 1 lane-per-column, 2 generic (test / A-B hook)
-int g_linearize_variant = getenv("HOP_LIN_VARIANT") ? atoi(getenv("HOP_LIN_VARIANT")) : 0;
+// quadrotor finite-difference kernel: 0 thread-per-step (default), 2 generic (test hook; identical bits)
+int g_linearize_variant = 0;
 
 template <int SYS>
 __global__ void k_rollout(int B, DynParams prm, int N, const double* __restrict__ x0, const double* __restrict__ U,
@@ -120,110 +118,20 @@ __device__ __noinline__ void quad_dynamics_cold(const double* p, const double* x
     dynamics<2>(p, x, u, xn);
 }
 
-// Quadrotor forward-difference linearisation (linearization.py:216-262), 16 lanes per (problem, step): lane c
-// perturbs coordinate c of (x, u).  Compared with the generic kernel above:
-//   * every lane evaluates ONE sincos (+ tan for the pitch lanes): lanes 0..2 the unperturbed roll / pitch / yaw,
-//     lanes 6..8 their perturbed angle; the unperturbed values reach the other lanes by shuffles (only an angle
-//     perturbation changes the trigonometry) -- same function values, so A and B are unchanged bit for bit;
-//   * f0 = F(X_k, U_k) is read from X[k+1] when the caller guarantees a consistent rollout (f0_from_x: the
-//     rollout / line-search kernels produced X with this very dynamics function), recomputed otherwise;
-//   * the 12 quotients (fp - f0) / h share one reciprocal: q0 = d * r, q = q0 + fma(-q0, h, d) * r, which is the
-//     correctly rounded quotient for r = RN(1/h) (Markstein), i.e. what the division returns.
-__global__ void __launch_bounds__(128) k_linearize_quad(int B, DynParams prm, int N, const double* __restrict__ X,
-                                                        const double* __restrict__ U, long ustride, double epsx, double epsu,
-                                                        double relx, double relu, int f0_from_x, const int* __restrict__ skip,
-                                                        double* __restrict__ A, double* __restrict__ Bm) {
-    constexpr int n = 12, m = 4, P = 16;
-    const size_t gid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const size_t total = (size_t)B * N * P;
-    const bool live = gid < total;
-    const size_t bk = live ? gid / P : 0;         // dead lanes shadow group 0 so that the shuffles stay converged
-    const int c = (int)(threadIdx.x & (P - 1));
-    const int k = (int)(bk % N);
-    const size_t b = bk / N;
-    const bool skipped = skip && skip[b];
-    double x[n], u[m];
-    const double* xs = X + (b * (N + 1) + k) * n;
-    const double* us = U + b * ustride + (size_t)k * m;
-#pragma unroll
-    for (int i = 0; i < n; ++i) x[i] = xs[i];
-#pragma unroll
-    for (int i = 0; i < m; ++i) u[i] = us[i];
-    // f0
-    double f0[n];
-    bool have_f0 = false;
-    if (f0_from_x) {
-        bool fin = true, finx = true;
-#pragma unroll
-        for (int i = 0; i < n; ++i) { f0[i] = xs[n + i]; fin = fin && isfinite(f0[i]); finx = finx && isfinite(x[i]); }
-        // X[k+1] non-finite although X[k] is finite: either F is non-finite there or the rollout cut the trajectory
-        // on its norm test (solver.py:57-59) -- only F itself can tell, so recompute
-        have_f0 = fin || !finx;
-    }
-    if (!have_f0) dynamics<2>(prm.p, x, u, f0);
-    bool nanout = false;
-#pragma unroll
-    for (int i = 0; i < n; ++i) nanout = nanout || !isfinite(f0[i]);      // linearization.py:243-248
-    // h = max(eps, rel * max(1, |v|))  (linearization.py:253,257)
-    double h = 0.0, base = 0.0;
-#pragma unroll
-    for (int i = 0; i < n; ++i) if (i == c) { base = x[i]; h = fmax(epsx, mul(relx, fmax(1.0, fabs(x[i])))); }
-#pragma unroll
-    for (int i = 0; i < m; ++i) if (i + n == c) { base = u[i]; h = fmax(epsu, mul(relu, fmax(1.0, fabs(u[i])))); }
-    const double vp = add(base, h);
-    // one angle per lane: lanes 6..8 their perturbed angle, everyone else the unperturbed angle (c mod 3)
-    const int role = (c >= 6 && c <= 8) ? c - 6 : c % 3;
-    const double ang = (c >= 6 && c <= 8) ? vp : (role == 0 ? x[6] : role == 1 ? x[7] : x[8]);
-    double sa, ca, ta = 0.0;
-    sincos(ang, &sa, &ca);
-    if (role == 1) ta = tan(ang);
-    QuadTrig T;
-    T.sph = __shfl_sync(0xffffffffu, sa, 0, P); T.cph = __shfl_sync(0xffffffffu, ca, 0, P);
-    T.sth = __shfl_sync(0xffffffffu, sa, 1, P); T.cth = __shfl_sync(0xffffffffu, ca, 1, P);
-    T.tth = __shfl_sync(0xffffffffu, ta, 1, P);
-    T.sps = __shfl_sync(0xffffffffu, sa, 2, P); T.cps = __shfl_sync(0xffffffffu, ca, 2, P);
-    if (c == 6) { T.sph = sa; T.cph = ca; }
-    if (c == 7) { T.sth = sa; T.cth = ca; T.tth = ta; }
-    if (c == 8) { T.sps = sa; T.cps = ca; }
-    if (!live || skipped) return;
-#pragma unroll
-    for (int i = 0; i < n; ++i) if (i == c) x[i] = vp;
-#pragma unroll
-    for (int i = 0; i < m; ++i) if (i + n == c) u[i] = vp;
-    double fp[n];
-    const bool bad = quad_guard(prm.p, x, u) || (fabs(T.cth) < prm.p[11]);
-    quad_core(prm.p, x, u, T, fp);
-    const double rh = 1.0 / h;
-    double col[n];
-#pragma unroll
-    for (int i = 0; i < n; ++i) {
-        const double d = sub(fp[i], f0[i]);
-        const double q0 = mul(d, rh);
-        const double q = fma(fma(-q0, h, d), rh, q0);
-        col[i] = (nanout || bad) ? nan("") : q;
-    }
-    if (c < n) {
-        double* Ak = A + bk * n * n;
-#pragma unroll
-        for (int i = 0; i < n; ++i) Ak[i * n + c] = col[i];
-    } else {
-        double* Bk = Bm + bk * n * m;
-#pragma unroll
-        for (int i = 0; i < n; ++i) Bk[i * m + (c - n)] = col[i];
-    }
-}
-
 // ---- quadrotor forward differences, ONE THREAD PER (problem, step) -----------------------------------------
-// k_linearize_quad above spends 1584 warp-instructions per 32 lanes (ncu: 80 % of them selects / moves / integer
-// tests that exist only because the perturbed coordinate is a run-time lane index).  Here the 16 perturbations are
-// a compile-time unrolled loop in one thread, so that
+// A lane-per-column mapping (16 lanes per (problem, step), lane c perturbs coordinate c) spent 1584 warp-instructions
+// per 32 lanes (ncu: 80 % of them selects / moves / integer tests that exist only because the perturbed coordinate is
+// a run-time lane index).  Here the 16 perturbations are a compile-time unrolled loop in one thread, so that
 //   * the perturbed evaluations share every sub-expression that does not depend on the perturbed coordinate
 //     (same operations on the same values -> same bits; the compiler's CSE does the sharing),
 //   * entries (i, c) whose output F_i does not depend on coordinate c are written as the exact 0.0 the reference
 //     obtains from (F_i - F_i) / h  (quad_affects below is the dependency structure of systems.py:170-210),
-//   * A_k and B_k are stored as full 32-byte sectors (four columns of a row at a time).
-// f0 = F(X_k, U_k) comes from X[k+1] (consistent rollout) or is evaluated; NaN / guard semantics as above.
-// Bit-identical to k_linearize<2> / k_linearize_quad (tests/test_gpu_parity.py compares them on random states).
+//   * A_k and B_k are stored as full 32-byte sectors (four columns of a row at a time),
+//   * the 12 quotients (fp - f0) / h of a column share one reciprocal: q0 = d * r, q = q0 + fma(-q0, h, d) * r, which
+//     is the correctly rounded quotient for r = RN(1/h) (Markstein), i.e. what the division returns.
+// f0 = F(X_k, U_k) is read from X[k+1] when the caller guarantees a consistent rollout (f0_from_x: the rollout /
+// line-search kernels produced X with this very dynamics function), evaluated otherwise; NaN / guard semantics as in
+// k_linearize.  Bit-identical to k_linearize<2> (tests/test_gpu_parity.py compares them on random states).
 // bit i of quad_affects(c): F_i depends on coordinate c of (x, u)
 __host__ __device__ constexpr unsigned quad_affects(int c) {
     return c == 0 ? 0x001u : c == 1 ? 0x002u : c == 2 ? 0x004u          // x, y, z        -> their own row
@@ -285,7 +193,8 @@ __device__ __forceinline__ void quad_fd_column(const double* p, const double* x0
     }
 }
 
-// MINB: CTAs per SM the register allocation is bounded for (3 -> 168 registers, 4 -> 128 with ~130 B of spills)
+// MINB: CTAs per SM the register allocation is bounded for (3 -> 168 registers; 4 -> 128 with ~130 B of spills was slower:
+// profiles/r1_experiments_overlap.txt)
 template <bool CENTRAL, int MINB = 3>
 __global__ void __launch_bounds__(128, MINB) k_linearize_quad_row(int B, DynParams prm, int N, const double* __restrict__ X,
                                                             const double* __restrict__ U, long ustride, double epsx, double epsu,
@@ -314,7 +223,9 @@ __global__ void __launch_bounds__(128, MINB) k_linearize_quad_row(int B, DynPara
             bool fin = true, finx = true;
 #pragma unroll
             for (int i = 0; i < n; ++i) { f0[i] = xs[n + i]; fin = fin && isfinite(f0[i]); finx = finx && isfinite(x[i]); }
-            have_f0 = fin || !finx;       // see k_linearize_quad
+            // X[k+1] non-finite although X[k] is finite: either F is non-finite there or the rollout cut the trajectory
+            // on its norm test (solver.py:57-59) -- only F itself can tell, so recompute
+            have_f0 = fin || !finx;
         }
         if (!have_f0) {                     // cold; through copies so that x, u, f0 themselves never live in local memory
             double xc[n], uc[m], fc[n];
@@ -398,22 +309,12 @@ static int launch_linearize(int B, const DynParams& prm, int N, const double* X,
     const size_t total = (size_t)B * N * P;
     const int threads = 128;
     const size_t grid = (total + threads - 1) / threads;
-    if (SYS == 2) {
-        // A/B + test switch: 0 (default) thread-per-step kernel, 1 lane-per-column kernel (forward only), 2 generic kernel
-        const int variant = g_linearize_variant;
-        if (variant == 0) {
-            const size_t rows = (size_t)B * N;
-            const unsigned g = (unsigned)((rows + threads - 1) / threads);
-            static const bool four = getenv("HOP_LIN_MINB") && atoi(getenv("HOP_LIN_MINB")) == 4;   // A/B switch
-            if (central) k_linearize_quad_row<true><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, 0, skip, A, Bm);
-            else if (four) k_linearize_quad_row<false, 4><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm);
-            else k_linearize_quad_row<false><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm);
-            return check_launch("k_linearize_quad_row");
-        }
-        if (variant == 1 && !central) {
-            k_linearize_quad<<<(unsigned)grid, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm);
-            return check_launch("k_linearize_quad");
-        }
+    if (SYS == 2 && g_linearize_variant == 0) {
+        const size_t rows = (size_t)B * N;
+        const unsigned g = (unsigned)((rows + threads - 1) / threads);
+        if (central) k_linearize_quad_row<true><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, 0, skip, A, Bm);
+        else k_linearize_quad_row<false><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm);
+        return check_launch("k_linearize_quad_row");
     }
     k_linearize<SYS><<<(unsigned)grid, threads, 0, st>>>(B, prm, N, X, U, ustride, central, epsx, epsu, relx, relu, skip, A, Bm);
     return check_launch("k_linearize");
