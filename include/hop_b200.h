@@ -58,7 +58,8 @@ enum { HOP_ST_OK = 0, HOP_ST_NONFINITE = 1, HOP_ST_LINALG = 2, HOP_ST_ERRMASK = 
  *          Tolerance on S2 (well conditioned): J within 1e-4 relative, T* reproduced on >= 99 % of instances (the
  *          mismatches are argmin gaps below the fp32 noise; measured in tests/ and DESIGN.md).  Not for the augmented
  *          problems: their 1e-9 jitter and 1e-12 regularisation are below fp32 resolution.
- *   VERIFIED: fused entry points and hop_ilqr_timeopt_f64 only (hop_select_f64 refuses it): FAST, then every instance whose
+ *   VERIFIED: fused entry points and hop_ilqr_timeopt_f64 (hop_select_f64 refuses it: at the LQR boundary the caller gives
+ *          the tolerance, hop_select_verified_f64): FAST, then every instance whose
  *          T* could depend on the implementation is recomputed in EXACT.  Per instance:
  *            1. the FAST selection, unchanged (same kernels, same routing, same bits);
  *            2. near-tie scan of the curve FAST returned (J_out, the curve the kernel minimised): with J1 = J(T*) and
@@ -109,7 +110,7 @@ int hop_device_count(void);
  * ((3,1) (4,2) (5,1) (12,4) (13,4)); HOP_MODE_EXACT and HOP_MODE_FP32 take any 1 <= d, m <= 16 */
 int hop_select_supported(int d, int m);
 /* same question for a given mode (HOP_MODE_VERIFIED: the FAST pairs whose state dimension n = d - 1 has a calibrated tie
- * tolerance, i.e. (3,1) and (13,4)) */
+ * tolerance, i.e. (3,1) and (13,4), for the fused forms; hop_select_verified_f64 takes every FAST pair) */
 int hop_select_supported_mode(int d, int m, int mode);
 
 /* horizon_selection.py:36-86 propagator_all_Jt_aug (+ solver.py:522,590 argmin), batched.
@@ -124,6 +125,35 @@ int hop_select_f64(int B, int N, int d, int m, int T_min, int T_max,
                    const double *A_aug, const double *B_aug, const double *Q_aug, const double *R_inv,
                    long rinv_step_stride, const double *z0, const double *QT, const double *w_explicit, int mode,
                    double *J_out, int *Tstar_out, double *Jstar_out, int *status, void *stream);
+
+/* HOP_MODE_VERIFIED at the LQR boundary, with a tie tolerance the CALLER chooses.  Arguments and outputs are those of
+ * hop_select_f64; `mode` is replaced by `tie_tol` (finite, > 0).  (d, m): the FAST pairs of hop_select_supported, else
+ * HOP_E_UNSUPPORTED_DIMS.  Argument errors are reported before any device is needed.  Per instance:
+ *   1. the FAST selection of hop_select_f64, unchanged (same routing and kernels, same bits);
+ *   2. the near-tie scan of HOP_MODE_VERIFIED on the curve the kernel minimised: v(t) = J(t) + w t, evaluated as
+ *      add_rn(J, mul_rn(w, t)) like the EXACT body, when w_explicit is given, J(t) otherwise; marked when the relative gap
+ *      is below tie_tol, when the window holds a NaN or +-Inf, when status != 0, or when the scan's argmin differs from
+ *      Tstar_out.  The pipelined FAST kernels (d = 12, 13) may contract J + w t into an FMA, so the last check also fires
+ *      on some last-bit differences of v: that only adds re-evaluations, it never hides a tie;
+ *   3. every marked instance is recomputed by the EXACT kernel (whole J_out row, Tstar_out, Jstar_out, status) and gets
+ *      HOP_ST_FLAG_REEVALUATED.
+ * T* and the low byte of status then equal HOP_MODE_EXACT's on every instance PROVIDED FAST stays within tie_tol / 2 of EXACT
+ * (relative, on v) at the competing horizons of the caller's input family.  The conditioning of LQR-boundary inputs belongs to
+ * the caller, so the library cannot fix one tolerance: choosing it is the caller's responsibility.  Deterministic; scratch of
+ * B + 1 ints, stream-ordered on `stream`; the host never waits.  Measured guidance (B200, tools/verified_ab.py,
+ * profiles/r4_verified_lqr_ab.jsonl; FAST's largest relative distance to EXACT on v at its two best horizons and at EXACT's T*):
+ *   S2 (tests/run_configs.py configuration 5: d = 4, 12, 13, N = 128, with w_explicit): distance <= 2.7e-14, so tie_tol = 1e-12
+ *     leaves an 18x margin on tie_tol / 2; at 1e-10 none of 262 144 (d = 4) / 65 536 (d = 12, 13) instances is re-evaluated and
+ *     VERIFIED takes FAST's time (d = 13: 51.4 ms against EXACT's 674 ms); 1e-7 would re-evaluate 0.02 %.
+ *   Quadrotor embedding built at the boundary (hop_build_augmented_f64 / hop_build_terminal_f64 on S1 linearisations, 16 384
+ *     instances): distance <= 4.7e-9; tie_tol = 1e-7 (10.7x margin) re-evaluates 2.8 %: FAST 16.2 ms, VERIFIED 34.3 ms,
+ *     EXACT 196 ms.  1e-8 would leave a margin of 1.07x.
+ *   Other families (ill-conditioned embeddings such as the cartpole's, see HOP_MODE_VERIFIED above): not measured;
+ *     measure FAST against EXACT on a sample of the family before choosing the tolerance. */
+int hop_select_verified_f64(int B, int N, int d, int m, int T_min, int T_max,
+                            const double *A_aug, const double *B_aug, const double *Q_aug, const double *R_inv,
+                            long rinv_step_stride, const double *z0, const double *QT, const double *w_explicit,
+                            double tie_tol, double *J_out, int *Tstar_out, double *Jstar_out, int *status, void *stream);
 
 /* Fused form: augmented.py:10-60 build_augmented_sequence_QR + augmented.py:63-87
  * build_terminal_aug_list + horizon_selection.py:36-86 + argmin in one kernel; the (n+1)^2 blocks are

@@ -1,4 +1,5 @@
 // hop_cabi.cu -- extern "C" surface of libhop_b200.so (see include/hop_b200.h for the contract).
+#include <cmath>
 #include <cstring>
 #include <mutex>
 #include <string>
@@ -65,6 +66,7 @@ int stream_alloc(void** ptr, size_t bytes, cudaStream_t st, const char* what);
 void stream_free(void* ptr, cudaStream_t st);
 int launch_scan_consts(int B, int d, int m, const double* R_inv1, double* R_inv, double* z0, cudaStream_t st);
 double verify_tie_tol(int n);
+int dispatch_select_generic_verified(int d, int m, double tol, const SelectArgs& p, cudaStream_t st);
 
 static thread_local std::string g_err;
 void set_last_error(const char* msg) { g_err = msg ? msg : ""; }
@@ -125,6 +127,27 @@ int hop_select_f64(int B, int N, int d, int m, int T_min, int T_max, const doubl
     SelectArgs p{B, N, T_min, T_max, kJitter, kMaxTries, A_aug, B_aug, Q_aug, R_inv, z0, QT, rinv_step_stride, w_explicit,
                  J_out, Tstar_out, Jstar_out, status, nullptr, nullptr, nullptr, g_generic_nodiag};
     return dispatch_select_generic(d, m, mode, p, (cudaStream_t)stream);
+}
+
+int hop_select_verified_f64(int B, int N, int d, int m, int T_min, int T_max, const double* A_aug, const double* B_aug,
+                            const double* Q_aug, const double* R_inv, long rinv_step_stride, const double* z0, const double* QT,
+                            const double* w_explicit, double tie_tol, double* J_out, int* Tstar_out, double* Jstar_out,
+                            int* status, void* stream) {
+    if (B < 0 || N < 1 || T_min < 1 || T_max < T_min || T_max > N || (rinv_step_stride != 0 && rinv_step_stride != (long)m * m) ||
+        !(std::isfinite(tie_tol) && tie_tol > 0.0)) {
+        set_last_error("hop_select_verified_f64: bad argument (need 1 <= T_min <= T_max <= N, rinv_step_stride in {0, m*m}, "
+                       "finite tie_tol > 0)");
+        return HOP_E_BADARG;
+    }
+    if (!hop_select_supported(d, m)) {
+        set_last_error("hop_select_verified_f64: (d, m) has no FAST kernel; supported: (3,1) (4,2) (5,1) (12,4) (13,4)");
+        return HOP_E_UNSUPPORTED_DIMS;
+    }
+    if (int rc = need_device()) return rc;
+    if (B == 0) return 0;
+    SelectArgs p{B, N, T_min, T_max, kJitter, kMaxTries, A_aug, B_aug, Q_aug, R_inv, z0, QT, rinv_step_stride, w_explicit,
+                 J_out, Tstar_out, Jstar_out, status, nullptr, nullptr, nullptr, g_generic_nodiag};
+    return dispatch_select_generic_verified(d, m, tie_tol, p, (cudaStream_t)stream);
 }
 
 int hop_select_fused_f64(int B, int N, int n, int m, int T_min, int T_max, const double* A, const double* Bm,

@@ -20,6 +20,7 @@
 // type: double, or float for HOP_MODE_FP32 (hop_select_f64 only; inputs are converted on load, J is written as double).
 #pragma once
 #include "hop_select_body.cuh"
+#include "../../include/hop_b200.h"
 
 namespace hop { namespace ref {
 
@@ -365,6 +366,19 @@ HOP_DEVICE void select_generic_body(const SelectArgs& p, int d, int m, int b, R*
         p.T_out[b] = am.idx;
         p.Jstar_out[b] = am.best;
         p.status[b] = flags | err;
+    }
+}
+
+// List mode of the LQR-boundary form (HOP_MODE_VERIFIED re-evaluation, fp64 only): this warp computes the instances
+// list[first], list[first + stride], ... below count, each exactly as select_generic_body computes it, and then sets
+// HOP_ST_FLAG_REEVALUATED in its status.  k_select_ref_generic passes its grid stride, the host emulation (0, 1).
+HOP_DEVICE void select_generic_list(const SelectArgs& p, int d, int m, const int* list, int count, int first, int stride,
+                                    double* s) {
+    for (int i = first; i < count; i += stride) {
+        const int b = list[i];
+        simt::sync();                                                             // the previous instance's slab reads are done
+        select_generic_body<double>(p, d, m, b, s);
+        if (simt::lane_id() == 0) p.status[b] |= HOP_ST_FLAG_REEVALUATED;
     }
 }
 

@@ -11,6 +11,10 @@
 // every lane ends with the same, order-independent result.  "Within the tolerance" is evaluated per horizon as
 // (J(t) - J1) / |J1| < tol with individually rounded operations: rounding is monotone, so some horizon passes exactly when
 // oracle/census.py argmin_gap (the same expression on the minimum over t != T*) is below tol.
+//
+// At the LQR boundary with an explicit time weight (hop_select_verified_f64, w_explicit given) the kernel minimised
+// v(t) = J(t) + w t while J_out holds the raw J(t); the scan then reads v(t) = add_rn(J(t), mul_rn(w, t)), the expression
+// (and the two roundings) of the EXACT body, so that the scan's argmin is EXACT's argmin on the same curve.
 #pragma once
 #include "hop_simt.cuh"
 
@@ -35,15 +39,18 @@ HOP_DEVICE bool argmin_takes(double v1, int t1, double v2, int t2) {
     return t2 < t1;
 }
 
-// warp-uniform: true when instance b is to be re-evaluated
-HOP_DEVICE bool tie_scan_warp(const TieScanArgs& a, int b) {
+// warp-uniform: true when instance b is to be re-evaluated.  w_explicit: null (the curve is J_out), or [B] (the curve is
+// J_out + w t).  A separate argument rather than a TieScanArgs field, so that the struct keeps its layout.
+HOP_DEVICE bool tie_scan_warp(const TieScanArgs& a, int b, const double* w_explicit = nullptr) {
     const int lane = simt::lane_id();
     const double* row = a.J + (size_t)b * a.T_max;
+    const double w = w_explicit ? w_explicit[b] : 0.0;
+    auto curve = [&](int t) { return w_explicit ? simt::add_rn(row[t - 1], simt::mul_rn(w, (double)t)) : row[t - 1]; };
     double best = 0.0;
     int tb = 0;
     bool nonfinite = false;
     for (int t = a.T_min + lane; t <= a.T_max; t += 32) {
-        const double v = row[t - 1];
+        const double v = curve(t);
         nonfinite = nonfinite || !isfinite(v);
         if (argmin_takes(best, tb, v, t)) { best = v; tb = t; }
     }
@@ -56,7 +63,7 @@ HOP_DEVICE bool tie_scan_warp(const TieScanArgs& a, int b) {
     if (!nonfinite) {            // (a lane that saw a non-finite value marks the instance anyway)
         const double scale = fabs(best);
         for (int t = a.T_min + lane; t <= a.T_max; t += 32)
-            if (t != tb) close = close || ((row[t - 1] - best) / scale < a.tol);
+            if (t != tb) close = close || ((curve(t) - best) / scale < a.tol);
     }
     const bool mark_here = nonfinite || close;
     return simt::ballot(mark_here) != 0u || a.status[b] != 0 || tb != a.T_star[b];

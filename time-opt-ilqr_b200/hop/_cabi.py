@@ -19,6 +19,7 @@ SIGNATURES = {
     "hop_select_supported": (_i, [_i, _i]),
     "hop_select_supported_mode": (_i, [_i, _i, _i]),
     "hop_select_f64": (_i, [_i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _l, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "hop_select_verified_f64": (_i, [_i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _l, _vp, _vp, _vp, _d, _vp, _vp, _vp, _vp, _vp]),
     "hop_select_fused_f64": (_i, [_i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _l, _vp, _vp, _vp, _vp, _vp, _vp, _u,
                                   _d, _d, _i, _vp, _vp, _vp, _vp, _vp]),
     "hop_rollout_f64": (_i, [_i, _i, _vp, _i, _vp, _vp, _l, _d, _vp, _vp]),

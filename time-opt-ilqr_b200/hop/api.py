@@ -13,6 +13,7 @@ provider); the work is done by libhop_b200.so through the C ABI in include/hop_b
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -31,7 +32,7 @@ MODE_GJ = 3      # materialised blocks + in-place Gauss-Jordan inverse with FMA 
 MODE_FP32 = 4    # propagator_all_Jt_aug_batched only: the EXACT sweep in single precision (well-conditioned problems only)
 MODE_VERIFIED = 5  # fused forms and the solver, quadrotor and DI: FAST, then instances whose two best horizons are within the
                    # measured tie tolerance (or with a non-finite window / non-zero status) recomputed in EXACT: T* and status low
-                   # byte equal EXACT's (include/hop_b200.h)
+                   # byte equal EXACT's (include/hop_b200.h); propagator_all_Jt_aug_batched with the caller's tie_tol
 ST_FLAG_REEVALUATED = 0x400   # include/hop_b200.h status bit 10: MODE_VERIFIED recomputed this instance in EXACT
 
 
@@ -112,9 +113,17 @@ def _outputs(B, T_max, device, want_J=True):
 
 
 def propagator_all_Jt_aug_batched(A_aug, B_aug, Q_aug, R_inv, z0, QT, T_min: int = 1, T_max: Optional[int] = None,
-                                  w_explicit=None, mode: int = MODE_EXACT) -> Selection:
+                                  w_explicit=None, mode: int = MODE_EXACT, tie_tol: Optional[float] = None) -> Selection:
     """Batched horizon_selection.propagator_all_Jt_aug + argmin.  Shapes: A_aug/Q_aug/QT [B,N,d,d],
-    B_aug [B,N,d,m], R_inv [B,m,m] or [m,m], z0 [B,d] or [d]."""
+    B_aug [B,N,d,m], R_inv [B,m,m] or [m,m], z0 [B,d] or [d].
+    mode=MODE_VERIFIED needs tie_tol (finite, > 0): the relative gap below which an instance's two best horizons count as
+    tied and the instance is recomputed in EXACT (hop_select_verified_f64).  T* equals EXACT's when FAST stays within
+    tie_tol / 2 of EXACT on the caller's inputs; include/hop_b200.h gives measured values per input family."""
+    if mode == MODE_VERIFIED:
+        if tie_tol is None or not math.isfinite(float(tie_tol)) or not float(tie_tol) > 0.0:
+            raise ValueError("mode=MODE_VERIFIED needs a finite tie_tol > 0 (the caller's tie tolerance, include/hop_b200.h)")
+    elif tie_tol is not None:
+        raise ValueError("tie_tol is only used with mode=MODE_VERIFIED")
     lib = _cabi.require_device()
     A_aug = _dev(A_aug)
     dev = A_aug.device
@@ -132,6 +141,12 @@ def propagator_all_Jt_aug_batched(A_aug, B_aug, Q_aug, R_inv, z0, QT, T_min: int
     wx = None if w_explicit is None else _dev(w_explicit, dev).reshape(Bsz)
     J, T, Js, st = _outputs(Bsz, T_max, dev)
     with torch.cuda.device(dev):
+        if mode == MODE_VERIFIED:
+            rc = lib.hop_select_verified_f64(Bsz, N, d, m, int(T_min), T_max, _ptr(A_aug), _ptr(B_aug), _ptr(Q_aug), _ptr(R_inv),
+                                             rstride, _ptr(z0), _ptr(QT), _ptr(wx), float(tie_tol), _ptr(J), _ptr(T), _ptr(Js),
+                                             _ptr(st), _stream(dev))
+            _cabi.check(rc, "hop_select_verified_f64")
+            return Selection(J, T, Js, st)
         rc = lib.hop_select_f64(Bsz, N, d, m, int(T_min), T_max, _ptr(A_aug), _ptr(B_aug), _ptr(Q_aug), _ptr(R_inv),
                                 rstride, _ptr(z0), _ptr(QT), _ptr(wx), mode, _ptr(J), _ptr(T), _ptr(Js), _ptr(st), _stream(dev))
     _cabi.check(rc, "hop_select_f64")

@@ -5,7 +5,8 @@
 
 Workloads: S1 (65 536 quadrotor selections, N = 128, the benchmark's seeding; selection on resident device inputs), the
 HOP-DDP configurations 2-4 of tests/run_configs.py, and a calibration pass of the small systems (DI, Segway, Cartpole through
-the three FAST routing branches): FAST's relative distance to EXACT at its two best horizons, and what the near-tie scan
+the three FAST routing branches) and, with --parts lqr, hop_select_verified_f64 at the LQR boundary (S2 as configuration 5
+generates it, and the quadrotor embedding materialised at the boundary): FAST's relative distance to EXACT at its two best horizons, and what the near-tie scan
 would decide at several tolerances (numpy restatement of include/hop_b200.h, HOP_MODE_VERIFIED step 2).  The modes are timed
 alternately (FAST, VERIFIED, EXACT per round) with CUDA events; the card's name and power limit are printed first.
 """
@@ -168,11 +169,103 @@ def ddp(args):
         emit(args.out, rec)
 
 
+LQR_TOLS = (1e-13, 1e-12, 1e-10, 1e-8, 1e-7)
+
+
+def s2_config5(B, d, m, N, seed=1234):
+    """S2 exactly as tests/run_configs.py configuration 5 generates a tile on the device (its first tile: seed 1234)."""
+    gen = torch.Generator(device=DEV); gen.manual_seed(seed)
+    A = torch.eye(d, dtype=torch.float64, device=DEV).expand(B, N, d, d) + \
+        0.05 / np.sqrt(d) * torch.randn((B, N, d, d), dtype=torch.float64, device=DEV, generator=gen)
+    Bm = 0.05 * torch.randn((B, N, d, m), dtype=torch.float64, device=DEV, generator=gen)
+    Q = torch.diag_embed(0.5 + 1.5 * torch.rand((B, N, d), dtype=torch.float64, device=DEV, generator=gen))
+    QT = (50.0 * torch.eye(d, dtype=torch.float64, device=DEV)).expand(B, N, d, d).contiguous()
+    Rd = 0.05 + 0.45 * torch.rand((B, m), dtype=torch.float64, device=DEV, generator=gen)
+    Rinv = torch.diag_embed(1.0 / (Rd + 1e-9))
+    z0 = torch.randn((B, d), dtype=torch.float64, device=DEV, generator=gen)
+    w = 0.01 + 0.09 * torch.rand((B,), dtype=torch.float64, device=DEV, generator=gen)
+    return (A, Bm, Q, Rinv, z0, QT), w
+
+
+def quad_embedding(B):
+    """S1 linearisations (the benchmark's seeding) materialised at the LQR boundary: hop_build_augmented_f64 /
+    hop_build_terminal_f64, R^-1 = chol_inv(sym(R)), z0 = e_d; the time weight is inside the blocks (no w_explicit)."""
+    import ctypes as C
+    import oracle as O
+    case = cases.make_case("Quadrotor", N=128)
+    F, x0, xg, u_ref, Q, R, alpha, w, N, T_min, T_max, wrap_idx, _ = case
+    n, m, d = 12, 4, 13
+    sel = api.HorizonSelector(case, B, device=DEV, mode=api.MODE_FAST)
+    sel(torch.as_tensor(s1_x0(B, seed=0), device=DEV))
+    X, A, Bm = sel.views()
+    t = lambda a: torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64), device=DEV)  # noqa: E731
+    A_aug = torch.empty((B, N, d, d), dtype=torch.float64, device=DEV); Q_aug = torch.empty_like(A_aug)
+    QT = torch.empty_like(A_aug); B_aug = torch.empty((B, N, d, m), dtype=torch.float64, device=DEV)
+    xg_t, w_t, ur_t, Q_t, Qf_t = t(np.broadcast_to(xg, (B, n))), t(np.full(B, float(w))), t(u_ref), t(Q), t(O.as_terminal_weight(alpha, n))
+    p_ = lambda a: C.c_void_p(a.data_ptr())  # noqa: E731
+    lib = api._cabi.require_device()
+    api._cabi.check(lib.hop_build_augmented_f64(B, N, n, m, p_(A), p_(Bm), None, p_(X), p_(sel.U), sel.ustride, p_(xg_t), p_(w_t),
+                                                p_(ur_t), p_(Q_t), O.wrap_mask(wrap_idx), 1e-9, 1e-12, p_(A_aug), p_(B_aug),
+                                                p_(Q_aug), None), "hop_build_augmented_f64")
+    api._cabi.check(lib.hop_build_terminal_f64(B, N, n, p_(X), p_(xg_t), p_(Qf_t), O.wrap_mask(wrap_idx), 1e-12, p_(QT), None),
+                    "hop_build_terminal_f64")
+    torch.cuda.synchronize()
+    z0 = np.zeros(d); z0[-1] = 1.0
+    return (A_aug, B_aug, Q_aug, t(O.chol_inv(0.5 * (R + R.T))), t(z0), QT), None, T_min, min(T_max, N)
+
+
+def lqr(args):
+    """hop_select_verified_f64 against FAST and EXACT at the LQR boundary: S2 as configuration 5 generates it (N = 128, with
+    w_explicit) and the quadrotor embedding materialised at the boundary.  Distances and scan shares are on the minimised
+    curve v = J + w t (J alone without w_explicit)."""
+    work = [("S2 d=4 m=2 N=128, w_explicit (configuration 5 generator)", lambda: (*s2_config5(262144, 4, 2, 128), 1, 128), args.s2_tol),
+            ("S2 d=12 m=4 N=128, w_explicit (configuration 5 generator)", lambda: (*s2_config5(65536, 12, 4, 128), 1, 128), args.s2_tol),
+            ("S2 d=13 m=4 N=128, w_explicit (configuration 5 generator)", lambda: (*s2_config5(65536, 13, 4, 128), 1, 128), args.s2_tol),
+            ("quadrotor embedding at the LQR boundary, 16384 S1 instances, N=128", lambda: quad_embedding(16384), args.quad_tol)]
+    for name, make, tol in work:
+        blocks, w, T_min, T_max = make()
+        B = blocks[0].shape[0]
+        def run(mode, blocks=blocks, w=w, T_min=T_min, T_max=T_max, tol=tol):
+            kw = {"tie_tol": tol} if mode == api.MODE_VERIFIED else {}
+            return api.propagator_all_Jt_aug_batched(*blocks, T_min, T_max, w_explicit=w, mode=mode, **kw)
+        ts = alternate({k: (lambda m=m: run(m)) for k, m in MODES.items()}, args.rounds)
+        out = {k: run(m) for k, m in MODES.items()}
+        torch.cuda.synchronize()
+        t = np.arange(1, T_max + 1, dtype=np.float64)
+        wn = np.zeros(B) if w is None else w.cpu().numpy()
+        V = {k: o.J.cpu().numpy() + wn[:, None] * t[None, :] for k, o in out.items()}       # numpy: two roundings, as the scan
+        Tf, Te = out["fast"].T_star.cpu().numpy().astype(np.int64), out["exact"].T_star.cpu().numpy().astype(np.int64)
+        rows = np.arange(B)
+        gap, second = census.argmin_gap(V["fast"], Tf, T_min, T_max)
+        r = lambda tt: np.abs(V["fast"][rows, tt - 1] - V["exact"][rows, tt - 1]) / np.abs(V["exact"][rows, tt - 1])  # noqa: E731
+        dist = np.maximum.reduce([r(Tf), r(second), r(Te)])
+        re = (out["verified"].status.cpu().numpy() & api.ST_FLAG_REEVALUATED) != 0
+        st = out["fast"].status.cpu().numpy()
+        s = summary(ts, B)
+        rec = {"workload": name, "card": args.card, "batch": B, "tie_tol": tol, "timing": s,
+               "verified_over_exact_throughput": s["verified"]["solves_per_s"] / s["exact"]["solves_per_s"],
+               "verified_over_fast_throughput": s["verified"]["solves_per_s"] / s["fast"]["solves_per_s"],
+               "reevaluated": int(re.sum()), "reevaluated_share": float(re.mean()),
+               "T_star_verified_ne_exact": int((out["verified"].T_star.cpu().numpy() != Te).sum()),
+               "T_star_fast_ne_exact": int((Tf != Te).sum()),
+               "max_rel_fast_vs_exact_at_candidates": float(dist.max()),
+               "p99_rel_fast_vs_exact_at_candidates": float(np.percentile(dist, 99)),
+               "max_fast_gap_where_T_differs": float(gap[Tf != Te].max()) if (Tf != Te).any() else None}
+        for tl in LQR_TOLS:
+            mark = scan_decision(V["fast"], Tf.astype(np.int32), st, T_min, T_max, tl)
+            rec[f"tol_{tl:g}"] = {"share": float(mark.mean()), "T_star_misses": int(((Tf != Te) & ~mark).sum())}
+        emit(args.out, rec)
+        del blocks, w, out, V
+        torch.cuda.empty_cache()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--out", default=None, help="also append the JSON lines to DIR/verified_ab.jsonl")
-    ap.add_argument("--parts", default="s1,small,ddp")
+    ap.add_argument("--parts", default="s1,small,ddp", help="any of s1, small, ddp, lqr")
+    ap.add_argument("--s2-tol", type=float, default=1e-10, help="tie_tol of the VERIFIED runs of the lqr part on S2")
+    ap.add_argument("--quad-tol", type=float, default=1e-7, help="tie_tol of the lqr part on the quadrotor embedding")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("verified_ab.py measures on the GPU; no CUDA device is visible")
@@ -187,6 +280,8 @@ def main():
         small_calibration(args)
     if "ddp" in parts:
         ddp(args)
+    if "lqr" in parts:
+        lqr(args)
 
 
 if __name__ == "__main__":
