@@ -8,8 +8,6 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.environ.get("HOP_BUILD_OUT") or os.path.join(os.path.dirname(HERE), "hop", "libhop_b200.so")   # experiments: other name
 SRCS = ["hop_select.cu", "hop_select_ref.cu", "hop_verify.cu", "hop_select_tpp.cu", "hop_select_epl.cu", "hop_traj.cu", "hop_ddp.cu", "hop_util.cu", "hop_cabi.cu"]
-HDRS = ["hop_simt.cuh", "hop_select_ref_body.cuh", "hop_verify_body.cuh", "hop_select_core.cuh", "hop_select_body.cuh", "hop_mma.cuh", "hop_select_mma_body.cuh", "hop_select_pipe_body.cuh", "hop_select_scan_body.cuh", "hop_select_gpipe_body.cuh", "hop_select_tpp_body.cuh", "hop_select_epl_body.cuh", "hop_dynamics.cuh", "hop_ddp_core.cuh", "hop_ddp_mma.cuh", "hop_common.cuh",
-        os.path.join("..", "..", "include", "hop_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
          "-Xptxas", "-v"] + os.environ.get("HOP_EXTRA_NVCC_FLAGS", "").split()
@@ -34,7 +32,9 @@ def includes_of(path, seen=None):
 
 
 def build(force=False, verbose=False):
-    deps = [os.path.join(HERE, f) for f in SRCS + HDRS]
+    deps = set()
+    for src in SRCS:
+        includes_of(os.path.join(HERE, src), deps)
     if not (force or stale(OUT, deps)):
         return OUT
 

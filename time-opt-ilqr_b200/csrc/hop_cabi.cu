@@ -10,64 +10,6 @@
 #include "../../include/hop_b200.h"
 
 namespace hop {
-int dispatch_select_generic(int d, int m, int mode, const SelectArgs& p, cudaStream_t st);
-long tpp_min_batch(long set_to);
-int dispatch_select_fused(int n, int m, const FusedArgs& p, cudaStream_t st);
-int dispatch_rollout(int B, int sys, const double* params_host, int N, const double* x0, const double* U, long ustride,
-                     double max_norm, double* X, cudaStream_t st);
-int dispatch_linearize(int B, int sys, const double* params_host, int N, const double* X, const double* U, long ustride,
-                       int central, double epsx, double epsu, double relx, double relu, int f0_from_x, const int* skip,
-                       double* A, double* Bm, cudaStream_t st);
-extern int g_linearize_variant;
-extern int g_backward_variant;
-extern int g_linesearch_variant;
-extern int g_fused_small_variant;
-extern int g_generic_pre;
-extern int g_generic_nodiag;
-struct DdpConst {
-    const double *xg, *w, *u_ref, *Q, *R, *Qf;
-    unsigned wrap_mask;
-};
-int dispatch_backward_linesearch(int sys, int B, const double* params_host, int N, const double* A, const double* Bm,
-                                 const double* X, const double* U, const DdpConst& c, const int* T, const double* lm,
-                                 const int* done, double* kl, double* Kl, int* ok, int* bw_err, double* Xn, double* Un,
-                                 double* Jn, int* acc, bool ordered, cudaEvent_t mid, cudaStream_t st);
-int dispatch_bruteforce(int n, int m, int B, int N, int T_max, const double* A, const double* Bm, const double* X, const double* U,
-                        long ustride, const DdpConst& c, double lm, double* J_out, int* status, cudaStream_t st);
-int dispatch_cost(int n, int m, int B, int N, const double* X, const double* U, const DdpConst& c, const int* T, double* J,
-                  cudaStream_t st);
-int dispatch_linesearch(int sys, int B, const double* params_host, int N, const double* X, const double* U, const DdpConst& c,
-                        const int* T, const double* kl, const double* Kl, const int* ok, double* Xn, double* Un, double* Jn,
-                        int* acc, cudaStream_t st);
-int launch_init_state(int B, double lm_init, double* lm, int* done, int* n_hist, int* status_out, cudaStream_t st);
-int launch_tile_u(int B, int N, int m, const double* u_ref, double* U, cudaStream_t st);
-int launch_after_select(int B, const int* sel_status, int* done, int* status_out, cudaStream_t st);
-int launch_warm_update(int B, int cap, const int* T_sel, const int* ok, const int* acc, const double* Jn, const int* bw_err,
-                       int* done, int* T_bar, double* J_hist, int* T_hist, int* n_hist, int* copy, int* status_out,
-                       cudaStream_t st);
-int launch_ddp_update(int B, int cap, const int* T_sel, const int* ok, const int* acc, const double* Jn, const int* bw_err,
-                      int* done, int* T_bar, double* lm, double* J_hist, int* T_hist, int* n_hist, int* copy,
-                      int* status_out, int* n_active, cudaStream_t st);
-int launch_copy_accepted(int B, size_t per_x, size_t per_u, const int* copy, const double* Xn, const double* Un, double* X,
-                         double* U, cudaStream_t st);
-int launch_finalize(int B, int cap, const int* n_hist, const int* T_hist, const int* T_bar, int* T_star, cudaStream_t st);
-int launch_chol(int B, int d, int c, const double* A, const double* Bm, double* X, double jitter, int max_tries, int* status,
-                cudaStream_t st);
-int launch_affine_residuals(int B, int sys, const double* params_host, int N, const double* X, const double* U, long ustride,
-                            double* a, cudaStream_t st);
-int launch_build_augmented(int B, int N, int n, int m, const double* A, const double* Bm, const double* a, const double* X,
-                           const double* U, long ustride, const double* xg, const double* w, const double* u_ref,
-                           const double* Q, unsigned wrap_mask, double q_reg, double rho_reg, double* A_aug, double* B_aug,
-                           double* Q_aug, cudaStream_t st);
-int launch_build_terminal(int B, int N, int n, const double* X, const double* xg, const double* Qf, unsigned wrap_mask,
-                          double rho_reg, double* QT, cudaStream_t st);
-int sys_dims(int sys, int* n, int* m);
-int stream_alloc(void** ptr, size_t bytes, cudaStream_t st, const char* what);
-void stream_free(void* ptr, cudaStream_t st);
-int launch_scan_consts(int B, int d, int m, const double* R_inv1, double* R_inv, double* z0, cudaStream_t st);
-double verify_tie_tol(int n);
-int dispatch_select_generic_verified(int d, int m, double tol, const SelectArgs& p, cudaStream_t st);
-
 static thread_local std::string g_err;
 void set_last_error(const char* msg) { g_err = msg ? msg : ""; }
 int report_cuda(cudaError_t e, const char* where) {
@@ -87,6 +29,56 @@ static int need_device() {
 }
 static const double kJitter = 1e-9;   // utils.py:69 defaults
 static const int kMaxTries = 8;
+
+namespace {
+// 1 <= T_min <= T_max <= N for a batch of B >= 0 instances, and R^-1 given per instance (stride 0) or per step (m * m)
+bool window_ok(int B, int N, int T_min, int T_max, long rinv_step_stride = 0, int m = 0) {
+    return B >= 0 && N >= 1 && T_min >= 1 && T_min <= T_max && T_max <= N &&
+           (rinv_step_stride == 0 || rinv_step_stride == (long)m * m);
+}
+
+// consecutive 256-byte-aligned regions of a caller's buffer; a null base only measures (the *_workspace_bytes queries)
+struct Carve {
+    char* base;
+    size_t off = 0;
+    template <typename T>
+    T* take(size_t count) {
+        char* q = base ? base + off : nullptr;
+        off += (sizeof(T) * count + 255) & ~(size_t)255;
+        return (T*)q;
+    }
+};
+
+// workspace of the x0 pipeline: X | A | Bm
+struct X0Ws {
+    double *X, *A, *Bm;
+    size_t total;
+};
+X0Ws x0_layout(char* base, int B, int N, int n, int m) {
+    Carve c{base};
+    X0Ws w;
+    w.X = c.take<double>((size_t)B * (N + 1) * n);
+    w.A = c.take<double>((size_t)B * N * n * n);
+    w.Bm = c.take<double>((size_t)B * N * n * m);
+    w.total = c.off;
+    return w;
+}
+
+// x0 -> T* on stream st: rollout (solver.py:42), forward-difference linearisation (linearization.py:177,216), fused selection
+int select_from_x0(int B, int sys, const double* params_host, int N, int n, int m, int T_min, int T_max, const double* x0,
+                   const double* U, long u_batch_stride, const double* xg, const double* w, const double* u_ref, const double* Q,
+                   const double* R, const double* Qf, unsigned wrap_mask, int central, int mode, const X0Ws& ws, double* J_out,
+                   int* Tstar_out, double* Jstar_out, int* status, cudaStream_t st) {
+    if (int rc = dispatch_rollout(B, sys, params_host, N, x0, U, u_batch_stride, 1e6, ws.X, st)) return rc;
+    // X comes from the rollout above, so F(X_k, U_k) = X[k+1] bit for bit: the linearisation may read f0 from it
+    if (int rc = dispatch_linearize(B, sys, params_host, N, ws.X, U, u_batch_stride, central, 1e-5, 1e-5, 1e-6, 1e-6, 1, nullptr,
+                                    ws.A, ws.Bm, st))
+        return rc;
+    // a_resid = NULL: on a trajectory produced by the rollout above F(X_k,U_k) - X_{k+1} is exactly 0
+    return hop_select_fused_f64(B, N, n, m, T_min, T_max, ws.A, ws.Bm, nullptr, ws.X, U, u_batch_stride, xg, w, u_ref, Q, R, Qf,
+                                wrap_mask, 1e-9, 1e-12, mode, J_out, Tstar_out, Jstar_out, status, st);
+}
+}  // namespace
 }  // namespace hop
 
 using namespace hop;
@@ -116,9 +108,7 @@ int hop_select_f64(int B, int N, int d, int m, int T_min, int T_max, const doubl
                    const double* Q_aug, const double* R_inv, long rinv_step_stride, const double* z0, const double* QT,
                    const double* w_explicit, int mode, double* J_out, int* Tstar_out, double* Jstar_out, int* status,
                    void* stream) {
-    if (B < 0 || N < 1 || T_min < 1 || T_max < T_min || T_max > N ||
-        mode < HOP_MODE_EXACT || mode > HOP_MODE_FP32 ||
-        (rinv_step_stride != 0 && rinv_step_stride != (long)m * m)) {
+    if (!window_ok(B, N, T_min, T_max, rinv_step_stride, m) || mode < HOP_MODE_EXACT || mode > HOP_MODE_FP32) {
         set_last_error("hop_select_f64: bad argument (need 1 <= T_min <= T_max <= N, rinv_step_stride in {0, m*m})");
         return HOP_E_BADARG;
     }
@@ -133,8 +123,7 @@ int hop_select_verified_f64(int B, int N, int d, int m, int T_min, int T_max, co
                             const double* Q_aug, const double* R_inv, long rinv_step_stride, const double* z0, const double* QT,
                             const double* w_explicit, double tie_tol, double* J_out, int* Tstar_out, double* Jstar_out,
                             int* status, void* stream) {
-    if (B < 0 || N < 1 || T_min < 1 || T_max < T_min || T_max > N || (rinv_step_stride != 0 && rinv_step_stride != (long)m * m) ||
-        !(std::isfinite(tie_tol) && tie_tol > 0.0)) {
+    if (!window_ok(B, N, T_min, T_max, rinv_step_stride, m) || !(std::isfinite(tie_tol) && tie_tol > 0.0)) {
         set_last_error("hop_select_verified_f64: bad argument (need 1 <= T_min <= T_max <= N, rinv_step_stride in {0, m*m}, "
                        "finite tie_tol > 0)");
         return HOP_E_BADARG;
@@ -156,42 +145,13 @@ int hop_select_fused_f64(int B, int N, int n, int m, int T_min, int T_max, const
                          const double* u_ref, const double* Q, const double* R, const double* Qf, unsigned wrap_mask,
                          double q_reg, double rho_reg, int mode, double* J_out, int* Tstar_out, double* Jstar_out,
                          int* status, void* stream) {
-    if (B < 0 || N < 1 || T_min < 1 || T_max < T_min || T_max > N || (mode != HOP_MODE_EXACT && mode != HOP_MODE_FAST && mode != HOP_MODE_GJ && mode != HOP_MODE_SCAN &&
-                                                                       mode != HOP_MODE_VERIFIED)) {
+    if (!window_ok(B, N, T_min, T_max) || (mode != HOP_MODE_EXACT && mode != HOP_MODE_FAST && mode != HOP_MODE_GJ &&
+                                          mode != HOP_MODE_SCAN && mode != HOP_MODE_VERIFIED)) {
         set_last_error("hop_select_fused_f64: bad argument (need 1 <= T_min <= T_max <= N, mode in {EXACT, FAST, GJ, SCAN, VERIFIED})");
         return HOP_E_BADARG;
     }
     if (int rc = need_device()) return rc;
     if (B == 0) return 0;
-    if (mode == HOP_MODE_SCAN) {
-        // the scan kernel works at the LQR boundary: materialise the augmented blocks (augmented.py:10-87) in a stream-ordered
-        // scratch allocation, then run the chunked parallel scan over the horizon.  Small batches only (that is where it pays).
-        if (!hop_select_supported_mode(n + 1, m, HOP_MODE_SCAN)) {
-            set_last_error("hop_select_fused_f64: HOP_MODE_SCAN is instantiated for (n, m) = (11,4) and (12,4) only");
-            return HOP_E_UNSUPPORTED_DIMS;
-        }
-        cudaStream_t st = (cudaStream_t)stream;
-        const int d = n + 1;
-        const size_t dd = (size_t)B * N * d * d, dm = (size_t)B * N * d * m;
-        const size_t total = sizeof(double) * (3 * dd + dm + (size_t)B * m * m + (size_t)B * d + (size_t)m * m) + sizeof(int);
-        void* ws = nullptr;
-        if (int rc = stream_alloc(&ws, total, st, "cudaMallocAsync(scan workspace)")) return rc;
-        double* A_aug = (double*)ws; double* Q_aug = A_aug + dd; double* QT = Q_aug + dd; double* B_aug = QT + dd;
-        double* R_inv = B_aug + dm; double* z0 = R_inv + (size_t)B * m * m; double* R1 = z0 + (size_t)B * d;
-        int* st1 = (int*)(R1 + m * m);
-        int rc = launch_build_augmented(B, N, n, m, A, Bm, a_resid, X, U, u_batch_stride, xg, w, u_ref, Q, wrap_mask, q_reg,
-                                        rho_reg, A_aug, B_aug, Q_aug, st);
-        if (!rc) rc = launch_build_terminal(B, N, n, X, xg, Qf, wrap_mask, rho_reg, QT, st);
-        if (!rc) rc = launch_chol(1, m, 0, R, nullptr, R1, kJitter, kMaxTries, st1, st);              // augmented.py:23
-        if (!rc) rc = launch_scan_consts(B, d, m, R1, R_inv, z0, st);                                 // augmented.py:59
-        if (!rc) {
-            SelectArgs q{B, N, T_min, T_max, kJitter, kMaxTries, A_aug, B_aug, Q_aug, R_inv, z0, QT, 0, nullptr,
-                         J_out, Tstar_out, Jstar_out, status, nullptr, nullptr, nullptr, g_generic_nodiag};
-            rc = dispatch_select_generic(d, m, HOP_MODE_SCAN, q, st);
-        }
-        stream_free(ws, st);
-        return rc;
-    }
     FusedArgs p{B, N, T_min, T_max, kJitter, kMaxTries, A, Bm, a_resid, X, U, u_batch_stride, xg, w, u_ref, Q, R, Qf,
                 wrap_mask, q_reg, rho_reg, mode, nullptr, J_out, Tstar_out, Jstar_out, status};
     return dispatch_select_fused(n, m, p, (cudaStream_t)stream);
@@ -215,13 +175,8 @@ int hop_linearize_f64(int B, int sys, const double* params_host, int N, const do
                               (cudaStream_t)stream);
 }
 
-static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-
 unsigned long long hop_select_from_x0_workspace_bytes(int B, int N, int n, int m) {
-    const size_t sX = align256(sizeof(double) * (size_t)B * (N + 1) * n);
-    const size_t sA = align256(sizeof(double) * (size_t)B * N * n * n);
-    const size_t sB = align256(sizeof(double) * (size_t)B * N * n * m);
-    return (unsigned long long)(sX + sA + sB);
+    return (unsigned long long)x0_layout(nullptr, B, N, n, m).total;
 }
 
 int hop_select_from_x0_f64(int B, int sys, const double* params_host, int N, int T_min, int T_max, const double* x0,
@@ -230,25 +185,17 @@ int hop_select_from_x0_f64(int B, int sys, const double* params_host, int N, int
                            int central, int mode, void* workspace, unsigned long long workspace_bytes, double* J_out,
                            int* Tstar_out, double* Jstar_out, int* status, void* stream) {
     int n = 0, m = 0;
-    if (sys_dims(sys, &n, &m)) { set_last_error("hop_select_from_x0_f64: unknown system id"); return HOP_E_BADARG; }
+    if (int rc = sys_dims(sys, "hop_select_from_x0_f64", &n, &m)) return rc;
     if (workspace_bytes < hop_select_from_x0_workspace_bytes(B, N, n, m) || (!workspace && B > 0)) {
         set_last_error("hop_select_from_x0_f64: workspace too small");
         return HOP_E_WORKSPACE;
     }
     if (B == 0) return 0;
-    char* ws = (char*)workspace;
-    double* X = (double*)ws;
-    double* A = (double*)(ws + align256(sizeof(double) * (size_t)B * (N + 1) * n));
-    double* Bm = (double*)((char*)A + align256(sizeof(double) * (size_t)B * N * n * n));
-    int rc = hop_rollout_f64(B, sys, params_host, N, x0, U, u_batch_stride, 1e6, X, stream);            // solver.py:42
-    if (rc) return rc;
-    // X comes from the rollout above, so F(X_k, U_k) = X[k+1] bit for bit: the linearisation may read f0 from it
-    rc = dispatch_linearize(B, sys, params_host, N, X, U, u_batch_stride, central, 1e-5, 1e-5, 1e-6, 1e-6, 1, nullptr, A, Bm,
-                            (cudaStream_t)stream);                                                       // linearization.py:177,216
-    if (rc) return rc;
-    // a_resid = NULL: on a trajectory produced by the rollout above F(X_k,U_k) - X_{k+1} is exactly 0
-    return hop_select_fused_f64(B, N, n, m, T_min, T_max, A, Bm, nullptr, X, U, u_batch_stride, xg, w, u_ref, Q, R, Qf,
-                                wrap_mask, 1e-9, 1e-12, mode, J_out, Tstar_out, Jstar_out, status, stream);
+    if (B < 0 || N < 1 || !params_host) { set_last_error("hop_select_from_x0_f64: bad argument"); return HOP_E_BADARG; }
+    if (int rc = need_device()) return rc;
+    return select_from_x0(B, sys, params_host, N, n, m, T_min, T_max, x0, U, u_batch_stride, xg, w, u_ref, Q, R, Qf, wrap_mask,
+                          central, mode, x0_layout((char*)workspace, B, N, n, m), J_out, Tstar_out, Jstar_out, status,
+                          (cudaStream_t)stream);
 }
 
 // ---- utilities of the reference API (utils.py, linearization.py:269, augmented.py) -----------------------
@@ -307,7 +254,7 @@ int hop_bruteforce_jt_f64(int B, int N, int n, int m, int T_max, const double* A
                           const double* U, long u_batch_stride, const double* xg, const double* w, const double* u_ref,
                           const double* Q, const double* R, const double* Qf, unsigned wrap_mask, double lm_lambda,
                           double* J_out, int* status, void* stream) {
-    if (B < 0 || N < 1 || T_max < 1 || T_max > N) { set_last_error("hop_bruteforce_jt_f64: need 1 <= T_max <= N"); return HOP_E_BADARG; }
+    if (!window_ok(B, N, 1, T_max)) { set_last_error("hop_bruteforce_jt_f64: need 1 <= T_max <= N"); return HOP_E_BADARG; }
     if (int rc = need_device()) return rc;
     if (B == 0) return 0;
     DdpConst c{xg, w, u_ref, Q, R, Qf, wrap_mask};
@@ -355,28 +302,27 @@ struct IlqrWs {
     size_t total;
 };
 IlqrWs ilqr_layout(char* base, int B, int N, int n, int m) {
+    Carve c{base};
     IlqrWs w;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { char* q = base ? base + off : nullptr; off += align256(bytes); return q; };
-    w.A = (double*)take(sizeof(double) * (size_t)B * N * n * n);
-    w.Bm = (double*)take(sizeof(double) * (size_t)B * N * n * m);
-    w.Xn = (double*)take(sizeof(double) * (size_t)B * (N + 1) * n);
-    w.Un = (double*)take(sizeof(double) * (size_t)B * N * m);
-    w.kl = (double*)take(sizeof(double) * (size_t)B * N * m);
-    w.Kl = (double*)take(sizeof(double) * (size_t)B * N * m * n);
-    w.lm = (double*)take(sizeof(double) * (size_t)B);
-    w.Jn = (double*)take(sizeof(double) * (size_t)B);
-    w.Jstar = (double*)take(sizeof(double) * (size_t)B);
-    w.T_bar = (int*)take(sizeof(int) * (size_t)B);
-    w.T_sel = (int*)take(sizeof(int) * (size_t)B);
-    w.ok = (int*)take(sizeof(int) * (size_t)B);
-    w.acc = (int*)take(sizeof(int) * (size_t)B);
-    w.bw_err = (int*)take(sizeof(int) * (size_t)B);
-    w.done = (int*)take(sizeof(int) * (size_t)B);
-    w.copy = (int*)take(sizeof(int) * (size_t)B);
-    w.sel_status = (int*)take(sizeof(int) * (size_t)B);
-    w.n_active = (int*)take(sizeof(int) * 4);
-    w.total = off;
+    w.A = c.take<double>((size_t)B * N * n * n);
+    w.Bm = c.take<double>((size_t)B * N * n * m);
+    w.Xn = c.take<double>((size_t)B * (N + 1) * n);
+    w.Un = c.take<double>((size_t)B * N * m);
+    w.kl = c.take<double>((size_t)B * N * m);
+    w.Kl = c.take<double>((size_t)B * N * m * n);
+    w.lm = c.take<double>(B);
+    w.Jn = c.take<double>(B);
+    w.Jstar = c.take<double>(B);
+    w.T_bar = c.take<int>(B);
+    w.T_sel = c.take<int>(B);
+    w.ok = c.take<int>(B);
+    w.acc = c.take<int>(B);
+    w.bw_err = c.take<int>(B);
+    w.done = c.take<int>(B);
+    w.copy = c.take<int>(B);
+    w.sel_status = c.take<int>(B);
+    w.n_active = c.take<int>(4);
+    w.total = c.off;
     return w;
 }
 }  // namespace
@@ -392,8 +338,8 @@ int hop_ilqr_timeopt_f64(int B, int sys, const double* params_host, int N, int T
                          double* J_hist, int* T_hist, int* n_hist, double* J_curve, int* T_star, int* status,
                          int* iters_run_host, double* timers_host, void* stream) {
     int n = 0, m = 0;
-    if (sys_dims(sys, &n, &m)) { set_last_error("hop_ilqr_timeopt_f64: unknown system id"); return HOP_E_BADARG; }
-    if (B < 0 || N < 1 || T_min < 1 || T_max < T_min || T_max > N || max_iter < 0 ||
+    if (int rc = sys_dims(sys, "hop_ilqr_timeopt_f64", &n, &m)) return rc;
+    if (!window_ok(B, N, T_min, T_max) || max_iter < 0 ||
         (mode != HOP_MODE_EXACT && mode != HOP_MODE_FAST && mode != HOP_MODE_GJ && mode != HOP_MODE_VERIFIED)) {
         set_last_error("hop_ilqr_timeopt_f64: bad argument (need 1 <= T_min <= T_max <= N, max_iter >= 0, mode in {EXACT, FAST, GJ, "
                        "VERIFIED})");
@@ -623,7 +569,7 @@ int hop_select_from_x0_host_f64(int B, int sys, const double* params_host, int N
                                 const double* Qf, unsigned wrap_mask, int central, int mode, double* J_out,
                                 int* Tstar_out, double* Jstar_out, int* status) {
     int n = 0, m = 0;
-    if (sys_dims(sys, &n, &m)) { set_last_error("hop_select_from_x0_host_f64: unknown system id"); return HOP_E_BADARG; }
+    if (int rc = sys_dims(sys, "hop_select_from_x0_host_f64", &n, &m)) return rc;
     if (int rc = need_device()) return rc;
     if (B <= 0) return B == 0 ? 0 : HOP_E_BADARG;
     std::lock_guard<std::mutex> lock(g_host.mu);
@@ -644,29 +590,33 @@ int hop_select_from_x0_host_f64(int B, int sys, const double* params_host, int N
     const int lanes = chunks > 1 ? 2 : 1;                         // workspaces (= streams) in use
     const bool shared_U = (u_batch_stride == 0);
     const size_t nU = shared_U ? (size_t)N * m : (size_t)B * N * m;
-    const size_t s_x0 = align256(sizeof(double) * (size_t)B * n), s_xg = s_x0, s_w = align256(sizeof(double) * (size_t)B);
-    const size_t s_U = align256(sizeof(double) * nU), s_c = align256(sizeof(double) * (size_t)(m + 2 * n * n + m * m));
-    const size_t s_J = align256(sizeof(double) * (size_t)B * T_max), s_T = align256(sizeof(int) * (size_t)B);
-    const size_t s_Js = align256(sizeof(double) * (size_t)B);
-    const size_t s_ws = align256((size_t)hop_select_from_x0_workspace_bytes(per, N, n, m));
-    const size_t total = s_x0 + s_xg + s_w + s_U + s_c + s_J + 2 * s_T + s_Js + lanes * s_ws;
+    // arena: x0 | xg | w | U | case constants | J | T* | status | J* | one x0-pipeline workspace per lane
+    const size_t s_ws = x0_layout(nullptr, per, N, n, m).total;
+    double *d_x0, *d_xg, *d_w, *d_U, *d_c, *d_J, *d_Js;
+    int *d_T, *d_st;
+    char* d_ws;
+    auto carve = [&](char* base) {
+        Carve a{base};
+        d_x0 = a.take<double>((size_t)B * n);
+        d_xg = a.take<double>((size_t)B * n);
+        d_w = a.take<double>(B);
+        d_U = a.take<double>(nU);
+        d_c = a.take<double>((size_t)(m + 2 * n * n + m * m));
+        d_J = a.take<double>((size_t)B * T_max);
+        d_T = a.take<int>(B);
+        d_st = a.take<int>(B);
+        d_Js = a.take<double>(B);
+        d_ws = a.take<char>(lanes * s_ws);
+        return a.off;
+    };
+    const size_t total = carve(nullptr);
     if (total > g_host.cap) {
         if (g_host.buf) cudaFree(g_host.buf);
         g_host.buf = nullptr; g_host.cap = 0;
         if (int rc = report_cuda(cudaMalloc(&g_host.buf, total), "cudaMalloc(host-variant arena)")) return rc;
         g_host.cap = total;
     }
-    char* q = (char*)g_host.buf;
-    double* d_x0 = (double*)q; q += s_x0;
-    double* d_xg = (double*)q; q += s_xg;
-    double* d_w = (double*)q; q += s_w;
-    double* d_U = (double*)q; q += s_U;
-    double* d_c = (double*)q; q += s_c;
-    double* d_J = (double*)q; q += s_J;
-    int* d_T = (int*)q; q += s_T;
-    int* d_st = (int*)q; q += s_T;
-    double* d_Js = (double*)q; q += s_Js;
-    char* d_ws = q;
+    carve((char*)g_host.buf);
     double* d_uref = d_c; double* d_Q = d_uref + m; double* d_R = d_Q + n * n; double* d_Qf = d_R + m * m;
     cudaStream_t s0 = g_host.stream[0];
     int rc = 0;
@@ -695,18 +645,9 @@ int hop_select_from_x0_host_f64(int B, int sys, const double* params_host, int N
             dU = d_U + o * N * m;
         }
         if (rc) break;
-        // workspace of this lane: X | A | Bm (hop_select_from_x0_workspace_bytes layout)
-        char* wsl = d_ws + lane * s_ws;
-        double* Xc = (double*)wsl;
-        double* Ac = (double*)(wsl + align256(sizeof(double) * (size_t)per * (N + 1) * n));
-        double* Bc = (double*)((char*)Ac + align256(sizeof(double) * (size_t)per * N * n * n));
-        if ((rc = dispatch_rollout(cb, sys, params_host, N, d_x0 + o * n, dU, u_batch_stride, 1e6, Xc, st))) break;         // solver.py:42
-        // X comes from the rollout above, so F(X_k, U_k) = X[k+1] bit for bit: the linearisation may read f0 from it
-        if ((rc = dispatch_linearize(cb, sys, params_host, N, Xc, dU, u_batch_stride, central, 1e-5, 1e-5, 1e-6, 1e-6, 1, nullptr,
-                                     Ac, Bc, st))) break;                                                                  // linearization.py:177,216
-        // a_resid = NULL: on a trajectory produced by the rollout above F(X_k,U_k) - X_{k+1} is exactly 0
-        rc = hop_select_fused_f64(cb, N, n, m, T_min, T_max, Ac, Bc, nullptr, Xc, dU, u_batch_stride, d_xg + o * n, d_w + o, d_uref,
-                                  d_Q, d_R, d_Qf, wrap_mask, 1e-9, 1e-12, mode, d_J + o * T_max, d_T + o, d_Js + o, d_st + o, st);
+        rc = select_from_x0(cb, sys, params_host, N, n, m, T_min, T_max, d_x0 + o * n, dU, u_batch_stride, d_xg + o * n, d_w + o,
+                            d_uref, d_Q, d_R, d_Qf, wrap_mask, central, mode, x0_layout(d_ws + lane * s_ws, per, N, n, m),
+                            d_J + o * T_max, d_T + o, d_Js + o, d_st + o, st);
         if (rc) break;
         if (J_out) copy(J_out + o * T_max, d_J + o * T_max, sizeof(double) * (size_t)cb * T_max, cudaMemcpyDeviceToHost, st, "D2H J");
         copy(Tstar_out + o, d_T + o, sizeof(int) * (size_t)cb, cudaMemcpyDeviceToHost, st, "D2H T*");

@@ -16,13 +16,6 @@
 
 namespace hop {
 
-struct DynParams2 { double p[HOP_NPARAMS]; };
-
-struct DdpConst {   // device pointers to the shared case constants + per-instance xg / w (mirrored in hop_cabi.cu)
-    const double *xg, *w, *u_ref, *Q, *R, *Qf;
-    unsigned wrap_mask;
-};
-
 // CostConst::diag for the whole CTA: the threads share the off-diagonal entries of Q, R, Qf (at most two loads each) and vote.
 // EVERY thread of the CTA calls this before any early return.
 template <int d>
@@ -168,7 +161,7 @@ int dispatch_bruteforce(int n, int m, int B, int N, int T_max, const double* A, 
 }
 
 template <int SYS>
-__global__ void k_linesearch(int B, DynParams2 prm, int N, const double* X, const double* U, DdpConst c, const int* T,
+__global__ void k_linesearch(int B, DynParams prm, int N, const double* X, const double* U, DdpConst c, const int* T,
                              const double* k_list, const double* K_list, const int* ok, const int* done, double* Xn,
                              double* Un, double* Jn, int* acc) {
     constexpr int n = SysDims<SYS>::n, m = SysDims<SYS>::m;
@@ -197,7 +190,7 @@ __global__ void k_linesearch(int B, DynParams2 prm, int N, const double* X, cons
 // HOP-DDP configurations leave the machine empty, so the extra threads are free).
 constexpr int kLsRoles = 6;
 template <int SYS>
-__global__ void __launch_bounds__(kLsRoles * 32) k_linesearch_par(int B, DynParams2 prm, int N, const double* X, const double* U,
+__global__ void __launch_bounds__(kLsRoles * 32) k_linesearch_par(int B, DynParams prm, int N, const double* X, const double* U,
                                                                     DdpConst c, const int* T, const double* k_list,
                                                                     const double* K_list, const int* ok, const int* done,
                                                                     double* Xn, double* Un, double* Jn, int* acc) {
@@ -250,7 +243,7 @@ __global__ void __launch_bounds__(kLsRoles * 32) k_linesearch_par(int B, DynPara
 // identical bits)
 int g_linesearch_variant = 0;
 template <int SYS>
-static int launch_linesearch(int B, const DynParams2& prm, int N, const double* X, const double* U, const DdpConst& c, const int* T,
+static int launch_linesearch(int B, const DynParams& prm, int N, const double* X, const double* U, const DdpConst& c, const int* T,
                              const double* kl, const double* Kl, const int* ok, const int* done, double* Xn, double* Un,
                              double* Jn, int* acc, cudaStream_t st) {
     const int threads = 64;
@@ -358,10 +351,8 @@ __global__ void k_tile_u(int B, int N, int m, const double* u_ref, double* U) {
     U[gid] = u_ref[gid % m];
 }
 
-static inline int grid1(size_t total, int threads) { return (int)((total + threads - 1) / threads); }
-
 template <int SYS>
-static int ddp_backward_linesearch(int B, const DynParams2& prm, int N, const double* A, const double* Bm, const double* X,
+static int ddp_backward_linesearch(int B, const DynParams& prm, int N, const double* A, const double* Bm, const double* X,
                                    const double* U, const DdpConst& c, const int* T, const double* lm, const int* done,
                                    double* kl, double* Kl, int* ok, int* bw_err, double* Xn, double* Un, double* Jn, int* acc,
                                    bool ordered, cudaEvent_t mid, cudaStream_t st) {
@@ -386,37 +377,20 @@ int dispatch_backward_linesearch(int sys, int B, const double* params_host, int 
                                  const double* X, const double* U, const DdpConst& c, const int* T, const double* lm,
                                  const int* done, double* kl, double* Kl, int* ok, int* bw_err, double* Xn, double* Un,
                                  double* Jn, int* acc, bool ordered, cudaEvent_t mid, cudaStream_t st) {
-    DynParams2 prm;
-    for (int i = 0; i < HOP_NPARAMS; ++i) prm.p[i] = params_host[i];
-    switch (sys) {
-        case 0: return ddp_backward_linesearch<0>(B, prm, N, A, Bm, X, U, c, T, lm, done, kl, Kl, ok, bw_err, Xn, Un, Jn, acc, ordered, mid, st);
-        case 1: return ddp_backward_linesearch<1>(B, prm, N, A, Bm, X, U, c, T, lm, done, kl, Kl, ok, bw_err, Xn, Un, Jn, acc, ordered, mid, st);
-        case 2: return ddp_backward_linesearch<2>(B, prm, N, A, Bm, X, U, c, T, lm, done, kl, Kl, ok, bw_err, Xn, Un, Jn, acc, ordered, mid, st);
-        case 3: return ddp_backward_linesearch<3>(B, prm, N, A, Bm, X, U, c, T, lm, done, kl, Kl, ok, bw_err, Xn, Un, Jn, acc, ordered, mid, st);
-    }
-    set_last_error("unknown system id");
-    return HOP_E_BADARG;
+    const DynParams prm = dyn_params(params_host);
+    return with_system(sys, "hop_backward_linesearch_f64", [&](auto s) {
+        return ddp_backward_linesearch<decltype(s)::value>(B, prm, N, A, Bm, X, U, c, T, lm, done, kl, Kl, ok, bw_err, Xn, Un, Jn,
+                                                           acc, ordered, mid, st);
+    });
 }
 
-template <int SYS>
-static int launch_linesearch_only(int B, const DynParams2& prm, int N, const double* X, const double* U, const DdpConst& c,
-                                  const int* T, const double* kl, const double* Kl, const int* ok, double* Xn, double* Un,
-                                  double* Jn, int* acc, cudaStream_t st) {
-    return launch_linesearch<SYS>(B, prm, N, X, U, c, T, kl, Kl, ok, nullptr, Xn, Un, Jn, acc, st);
-}
 int dispatch_linesearch(int sys, int B, const double* params_host, int N, const double* X, const double* U, const DdpConst& c,
                         const int* T, const double* kl, const double* Kl, const int* ok, double* Xn, double* Un, double* Jn,
                         int* acc, cudaStream_t st) {
-    DynParams2 prm;
-    for (int i = 0; i < HOP_NPARAMS; ++i) prm.p[i] = params_host[i];
-    switch (sys) {
-        case 0: return launch_linesearch_only<0>(B, prm, N, X, U, c, T, kl, Kl, ok, Xn, Un, Jn, acc, st);
-        case 1: return launch_linesearch_only<1>(B, prm, N, X, U, c, T, kl, Kl, ok, Xn, Un, Jn, acc, st);
-        case 2: return launch_linesearch_only<2>(B, prm, N, X, U, c, T, kl, Kl, ok, Xn, Un, Jn, acc, st);
-        case 3: return launch_linesearch_only<3>(B, prm, N, X, U, c, T, kl, Kl, ok, Xn, Un, Jn, acc, st);
-    }
-    set_last_error("unknown system id");
-    return HOP_E_BADARG;
+    const DynParams prm = dyn_params(params_host);
+    return with_system(sys, "hop_linesearch_f64", [&](auto s) {
+        return launch_linesearch<decltype(s)::value>(B, prm, N, X, U, c, T, kl, Kl, ok, nullptr, Xn, Un, Jn, acc, st);
+    });
 }
 
 int dispatch_cost(int n, int m, int B, int N, const double* X, const double* U, const DdpConst& c, const int* T, double* J,

@@ -256,19 +256,6 @@ static int launch_fused_mma(const FusedArgs& p, cudaStream_t st) {
     return check_launch("k_select_fused_mma");
 }
 
-
-// one problem per THREAD (d <= 5, large batches): hop_select_tpp.cu.  Returns HOP_E_UNSUPPORTED_DIMS without touching the
-// error string when (d, m, p) is not for that kernel.
-int dispatch_select_generic_tpp(int d, int m, const SelectArgs& p, cudaStream_t st);
-// one matrix element per LANE, fused form of the small systems: hop_select_epl.cu (same convention)
-int dispatch_select_fused_epl(int n, int m, const FusedArgs& p, cudaStream_t st);
-
-// HOP_MODE_EXACT / HOP_MODE_FP32: reference operation order, hop_select_ref.cu
-int dispatch_select_ref_generic(int d, int m, bool fp32, const SelectArgs& p, cudaStream_t st);
-int dispatch_select_ref_fused(int n, int m, const FusedArgs& p, cudaStream_t st);
-// HOP_MODE_VERIFIED: FAST, near-tie scan, EXACT on the marked instances (hop_verify.cu)
-int dispatch_select_verified(int n, int m, const FusedArgs& p, cudaStream_t st);
-
 int dispatch_select_generic(int d, int m, int mode, const SelectArgs& p, cudaStream_t st) {
     if (mode == HOP_MODE_EXACT || mode == HOP_MODE_FP32) return dispatch_select_ref_generic(d, m, mode == HOP_MODE_FP32, p, st);
     if (mode == HOP_MODE_SCAN) {
@@ -290,8 +277,39 @@ int dispatch_select_generic(int d, int m, int mode, const SelectArgs& p, cudaStr
     return HOP_E_UNSUPPORTED_DIMS;
 }
 
+// HOP_MODE_SCAN of the fused form: the scan kernel works at the LQR boundary, so materialise the augmented blocks
+// (augmented.py:10-87) in a stream-ordered scratch allocation, then run the chunked parallel scan over the horizon.  Small
+// batches only (that is where it pays).
+static int select_fused_scan(int n, int m, const FusedArgs& p, cudaStream_t st) {
+    if (!hop_select_supported_mode(n + 1, m, HOP_MODE_SCAN)) {
+        set_last_error("hop_select_fused_f64: HOP_MODE_SCAN is instantiated for (n, m) = (11,4) and (12,4) only");
+        return HOP_E_UNSUPPORTED_DIMS;
+    }
+    const int B = p.B, N = p.N, d = n + 1;
+    const size_t dd = (size_t)B * N * d * d, dm = (size_t)B * N * d * m;
+    const size_t total = sizeof(double) * (3 * dd + dm + (size_t)B * m * m + (size_t)B * d + (size_t)m * m) + sizeof(int);
+    void* ws = nullptr;
+    if (int rc = stream_alloc(&ws, total, st, "cudaMallocAsync(scan workspace)")) return rc;
+    double* A_aug = (double*)ws; double* Q_aug = A_aug + dd; double* QT = Q_aug + dd; double* B_aug = QT + dd;
+    double* R_inv = B_aug + dm; double* z0 = R_inv + (size_t)B * m * m; double* R1 = z0 + (size_t)B * d;
+    int* st1 = (int*)(R1 + m * m);
+    int rc = launch_build_augmented(B, N, n, m, p.A, p.Bm, p.a_resid, p.X, p.U, p.u_stride, p.xg, p.w, p.u_ref, p.Q, p.wrap_mask,
+                                    p.q_reg, p.rho_reg, A_aug, B_aug, Q_aug, st);
+    if (!rc) rc = launch_build_terminal(B, N, n, p.X, p.xg, p.Qf, p.wrap_mask, p.rho_reg, QT, st);
+    if (!rc) rc = launch_chol(1, m, 0, p.R, nullptr, R1, p.jitter, p.max_tries, st1, st);          // augmented.py:23
+    if (!rc) rc = launch_scan_consts(B, d, m, R1, R_inv, z0, st);                                 // augmented.py:59
+    if (!rc) {
+        SelectArgs q{B, N, p.T_min, p.T_max, p.jitter, p.max_tries, A_aug, B_aug, Q_aug, R_inv, z0, QT, 0, nullptr,
+                     p.J_out, p.T_out, p.Jstar_out, p.status, nullptr, nullptr, nullptr, g_generic_nodiag};
+        rc = dispatch_select_generic(d, m, HOP_MODE_SCAN, q, st);
+    }
+    stream_free(ws, st);
+    return rc;
+}
+
 int dispatch_select_fused(int n, int m, const FusedArgs& p, cudaStream_t st) {
-    if (p.mode == HOP_MODE_EXACT) return dispatch_select_ref_fused(n, m, p, st);
+    if (p.mode == HOP_MODE_SCAN) return select_fused_scan(n, m, p, st);
+    if (p.mode == HOP_MODE_EXACT) return launch_ref_fused_list(n, m, p, nullptr, nullptr, st);
     if (p.mode == HOP_MODE_VERIFIED) return dispatch_select_verified(n, m, p, st);
     if (n <= 4) {
         const int rc = dispatch_select_fused_epl(n, m, p, st);

@@ -148,8 +148,4 @@ int launch_ref_fused_list(int n, int m, const FusedArgs& p, const int* list, con
     return check_launch("k_select_ref_fused");
 }
 
-int dispatch_select_ref_fused(int n, int m, const FusedArgs& p, cudaStream_t st) {
-    return launch_ref_fused_list(n, m, p, nullptr, nullptr, st);
-}
-
 }  // namespace hop

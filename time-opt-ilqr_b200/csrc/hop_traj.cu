@@ -10,8 +10,6 @@
 
 namespace hop {
 
-struct DynParams { double p[HOP_NPARAMS]; };
-
 // quadrotor finite-difference kernel: 0 thread-per-step (default), 2 generic (test hook; identical bits)
 int g_linearize_variant = 0;
 
@@ -294,69 +292,44 @@ __global__ void __launch_bounds__(128, MINB) k_linearize_quad_row(int B, DynPara
 #undef HOP_FD4
 }
 
-template <int SYS>
-static int launch_rollout(int B, const DynParams& prm, int N, const double* x0, const double* U, long ustride,
-                          double max_norm, double* X, cudaStream_t st) {
-    const int threads = 128;
-    k_rollout<SYS><<<(B + threads - 1) / threads, threads, 0, st>>>(B, prm, N, x0, U, ustride, max_norm, X);
-    return check_launch("k_rollout");
-}
-template <int SYS>
-static int launch_linearize(int B, const DynParams& prm, int N, const double* X, const double* U, long ustride,
-                            int central, double epsx, double epsu, double relx, double relu, int f0_from_x, const int* skip,
-                            double* A, double* Bm, cudaStream_t st) {
-    constexpr int P = SysDims<SYS>::n + SysDims<SYS>::m;
-    const size_t total = (size_t)B * N * P;
-    const int threads = 128;
-    const size_t grid = (total + threads - 1) / threads;
-    if (SYS == 2 && g_linearize_variant == 0) {
-        const size_t rows = (size_t)B * N;
-        const unsigned g = (unsigned)((rows + threads - 1) / threads);
-        if (central) k_linearize_quad_row<true><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, 0, skip, A, Bm);
-        else k_linearize_quad_row<false><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm);
-        return check_launch("k_linearize_quad_row");
-    }
-    k_linearize<SYS><<<(unsigned)grid, threads, 0, st>>>(B, prm, N, X, U, ustride, central, epsx, epsu, relx, relu, skip, A, Bm);
-    return check_launch("k_linearize");
-}
-
 int dispatch_rollout(int B, int sys, const double* params_host, int N, const double* x0, const double* U, long ustride,
                      double max_norm, double* X, cudaStream_t st) {
-    DynParams prm;
-    for (int i = 0; i < HOP_NPARAMS; ++i) prm.p[i] = params_host[i];
-    switch (sys) {
-        case 0: return launch_rollout<0>(B, prm, N, x0, U, ustride, max_norm, X, st);
-        case 1: return launch_rollout<1>(B, prm, N, x0, U, ustride, max_norm, X, st);
-        case 2: return launch_rollout<2>(B, prm, N, x0, U, ustride, max_norm, X, st);
-        case 3: return launch_rollout<3>(B, prm, N, x0, U, ustride, max_norm, X, st);
-    }
-    set_last_error("hop_rollout_f64: unknown system id");
-    return HOP_E_BADARG;
+    const DynParams prm = dyn_params(params_host);
+    return with_system(sys, "hop_rollout_f64", [&](auto s) {
+        const int threads = 128;
+        k_rollout<decltype(s)::value><<<(B + threads - 1) / threads, threads, 0, st>>>(B, prm, N, x0, U, ustride, max_norm, X);
+        return check_launch("k_rollout");
+    });
 }
 
 int dispatch_linearize(int B, int sys, const double* params_host, int N, const double* X, const double* U, long ustride,
                        int central, double epsx, double epsu, double relx, double relu, int f0_from_x, const int* skip,
                        double* A, double* Bm, cudaStream_t st) {
-    DynParams prm;
-    for (int i = 0; i < HOP_NPARAMS; ++i) prm.p[i] = params_host[i];
-    switch (sys) {
-        case 0: return launch_linearize<0>(B, prm, N, X, U, ustride, central, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm, st);
-        case 1: return launch_linearize<1>(B, prm, N, X, U, ustride, central, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm, st);
-        case 2: return launch_linearize<2>(B, prm, N, X, U, ustride, central, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm, st);
-        case 3: return launch_linearize<3>(B, prm, N, X, U, ustride, central, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm, st);
-    }
-    set_last_error("hop_linearize_f64: unknown system id");
-    return HOP_E_BADARG;
+    const DynParams prm = dyn_params(params_host);
+    return with_system(sys, "hop_linearize_f64", [&](auto s) {
+        constexpr int SYS = decltype(s)::value;
+        constexpr int P = SysDims<SYS>::n + SysDims<SYS>::m;
+        const size_t total = (size_t)B * N * P;
+        const int threads = 128;
+        const size_t grid = (total + threads - 1) / threads;
+        if (SYS == 2 && g_linearize_variant == 0) {
+            const size_t rows = (size_t)B * N;
+            const unsigned g = (unsigned)((rows + threads - 1) / threads);
+            if (central) k_linearize_quad_row<true><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, 0, skip, A, Bm);
+            else k_linearize_quad_row<false><<<g, threads, 0, st>>>(B, prm, N, X, U, ustride, epsx, epsu, relx, relu, f0_from_x, skip, A, Bm);
+            return check_launch("k_linearize_quad_row");
+        }
+        k_linearize<SYS><<<(unsigned)grid, threads, 0, st>>>(B, prm, N, X, U, ustride, central, epsx, epsu, relx, relu, skip, A, Bm);
+        return check_launch("k_linearize");
+    });
 }
 
-int sys_dims(int sys, int* n, int* m) {
-    switch (sys) {
-        case 0: *n = 2; *m = 1; return 0;
-        case 1: *n = 4; *m = 1; return 0;
-        case 2: *n = 12; *m = 4; return 0;
-        case 3: *n = 4; *m = 1; return 0;
-    }
-    return HOP_E_BADARG;
+int sys_dims(int sys, const char* where, int* n, int* m) {
+    return with_system(sys, where, [&](auto s) {
+        *n = SysDims<decltype(s)::value>::n;
+        *m = SysDims<decltype(s)::value>::m;
+        return 0;
+    });
 }
 
 }  // namespace hop

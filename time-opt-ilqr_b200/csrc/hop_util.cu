@@ -110,10 +110,8 @@ __global__ void k_chol(int B, int d, int c, const double* A, const double* Bm, d
     status[b] = st;
 }
 
-struct DynParams3 { double p[HOP_NPARAMS]; };
-
 template <int SYS>
-__global__ void k_affine_residuals(int B, DynParams3 prm, int N, const double* X, const double* U, long ustride, double* a) {
+__global__ void k_affine_residuals(int B, DynParams prm, int N, const double* X, const double* U, long ustride, double* a) {
     constexpr int n = SysDims<SYS>::n, m = SysDims<SYS>::m;
     const size_t gid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (gid >= (size_t)B * N) return;
@@ -206,43 +204,36 @@ __global__ void k_scan_consts(int B, int d, int m, const double* R_inv1, double*
     if (gid < nz) z0[gid] = ((int)(gid % d) == d - 1) ? 1.0 : 0.0;
 }
 
-static inline int grid1u(size_t total, int threads) { return (int)((total + threads - 1) / threads); }
-
 int launch_chol(int B, int d, int c, const double* A, const double* Bm, double* X, double jitter, int max_tries, int* status,
                 cudaStream_t st) {
-    k_chol<<<grid1u(B, 64), 64, 0, st>>>(B, d, c, A, Bm, X, jitter, max_tries, status);
+    k_chol<<<grid1(B, 64), 64, 0, st>>>(B, d, c, A, Bm, X, jitter, max_tries, status);
     return check_launch("k_chol");
 }
 int launch_scan_consts(int B, int d, int m, const double* R_inv1, double* R_inv, double* z0, cudaStream_t st) {
     const size_t total = (size_t)B * (m * m > d ? m * m : d);
-    k_scan_consts<<<grid1u(total, 128), 128, 0, st>>>(B, d, m, R_inv1, R_inv, z0);
+    k_scan_consts<<<grid1(total, 128), 128, 0, st>>>(B, d, m, R_inv1, R_inv, z0);
     return check_launch("k_scan_consts");
 }
 int launch_affine_residuals(int B, int sys, const double* params_host, int N, const double* X, const double* U, long ustride,
                             double* a, cudaStream_t st) {
-    DynParams3 prm;
-    for (int i = 0; i < HOP_NPARAMS; ++i) prm.p[i] = params_host[i];
-    const int g = grid1u((size_t)B * N, 128);
-    switch (sys) {
-        case 0: k_affine_residuals<0><<<g, 128, 0, st>>>(B, prm, N, X, U, ustride, a); break;
-        case 1: k_affine_residuals<1><<<g, 128, 0, st>>>(B, prm, N, X, U, ustride, a); break;
-        case 2: k_affine_residuals<2><<<g, 128, 0, st>>>(B, prm, N, X, U, ustride, a); break;
-        case 3: k_affine_residuals<3><<<g, 128, 0, st>>>(B, prm, N, X, U, ustride, a); break;
-        default: set_last_error("unknown system id"); return HOP_E_BADARG;
-    }
-    return check_launch("k_affine_residuals");
+    const DynParams prm = dyn_params(params_host);
+    const int g = grid1((size_t)B * N, 128);
+    return with_system(sys, "hop_affine_residuals_f64", [&](auto s) {
+        k_affine_residuals<decltype(s)::value><<<g, 128, 0, st>>>(B, prm, N, X, U, ustride, a);
+        return check_launch("k_affine_residuals");
+    });
 }
 int launch_build_augmented(int B, int N, int n, int m, const double* A, const double* Bm, const double* a, const double* X,
                            const double* U, long ustride, const double* xg, const double* w, const double* u_ref,
                            const double* Q, unsigned wrap_mask, double q_reg, double rho_reg, double* A_aug, double* B_aug,
                            double* Q_aug, cudaStream_t st) {
-    k_build_augmented<<<grid1u((size_t)B * N, 128), 128, 0, st>>>(B, N, n, m, A, Bm, a, X, U, ustride, xg, w, u_ref, Q, wrap_mask,
+    k_build_augmented<<<grid1((size_t)B * N, 128), 128, 0, st>>>(B, N, n, m, A, Bm, a, X, U, ustride, xg, w, u_ref, Q, wrap_mask,
                                                                  q_reg, rho_reg, A_aug, B_aug, Q_aug);
     return check_launch("k_build_augmented");
 }
 int launch_build_terminal(int B, int N, int n, const double* X, const double* xg, const double* Qf, unsigned wrap_mask,
                           double rho_reg, double* QT, cudaStream_t st) {
-    k_build_terminal<<<grid1u((size_t)B * N, 128), 128, 0, st>>>(B, N, n, X, xg, Qf, wrap_mask, rho_reg, QT);
+    k_build_terminal<<<grid1((size_t)B * N, 128), 128, 0, st>>>(B, N, n, X, xg, Qf, wrap_mask, rho_reg, QT);
     return check_launch("k_build_terminal");
 }
 

@@ -9,13 +9,6 @@
 
 namespace hop {
 
-int dispatch_select_fused(int n, int m, const FusedArgs& p, cudaStream_t st);
-int dispatch_select_generic(int d, int m, int mode, const SelectArgs& p, cudaStream_t st);
-int launch_ref_fused_list(int n, int m, const FusedArgs& p, const int* list, const int* list_count, cudaStream_t st);
-int launch_ref_generic_list(int d, int m, const SelectArgs& p, const int* list, const int* list_count, cudaStream_t st);
-int stream_alloc(void** ptr, size_t bytes, cudaStream_t st, const char* what);
-void stream_free(void* ptr, cudaStream_t st);
-
 constexpr int kScanWarps = 8;
 
 // w_explicit: null, or [B] at the LQR boundary (the scanned curve is then J + w t, hop_verify_body.cuh)
